@@ -10,6 +10,8 @@ reference keeps that state in PostgreSQL between its `digest` and `identificatio
   python bench.py --impl reference [...]                     the CPU arm: the oracle port of the reference's
                                                              algorithm on the host cores (the Rust reference cannot be
                                                              built here: no cargo/PostgreSQL/Comet)
+  python bench.py [...] --dump-outputs DIR                   also write the PSM table of the last timed step as
+                                                             DIR/<field>.npy, to compare two builds output for output
 N > 1 is launched by torchrun (one rank per GPU).  The headline value is weak scaling (every rank searches its own
 10k-spectrum batch of the C2 workload, index replicated); the PSM tables are gathered by the library itself
 (md_comm_init / md_gather_psms: NCCL on the library's comm stream).  The same run also measures C4 -- ONE fixed set of
@@ -146,6 +148,34 @@ def psm_crc(table):
     return zlib.crc32(np.ascontiguousarray(table).tobytes()) & 0xFFFFFFFF
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(table, out_dir):
+    """Write a PSM table [spectra, top_k] as one .npy per field.  Integer fields are stored as float64 (checked exact),
+    var_mask (a 64-bit position mask) as its two 32-bit halves, score as float32.  Tables larger than DUMP_BYTES are
+    cut to a fixed, seeded sample of spectra; `spectrum_row.npy` holds the rows kept."""
+    import numpy as np
+    ints = [f for f in table.dtype.names if f not in ("_pad", "var_mask", "score")]
+    per_spectrum = table.shape[1] * (8 * (len(ints) + 2) + 4) + 8
+    keep = (DUMP_BYTES - 256 * (len(ints) + 4)) // per_spectrum      # 256: room for each file's .npy header
+    n = table.shape[0]
+    rows = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    sub = table[rows]
+    vm = sub["var_mask"]
+    out = {f: sub[f].astype(np.float64) for f in ints}
+    out["var_mask_lo32"] = (vm & np.uint64(0xFFFFFFFF)).astype(np.float64)
+    out["var_mask_hi32"] = (vm >> np.uint64(32)).astype(np.float64)
+    out["score"] = sub["score"].astype(np.float32)
+    out["spectrum_row"] = rows.astype(np.float64)
+    for f in ints:
+        if not np.array_equal(out[f].astype(sub[f].dtype), sub[f]):
+            raise ValueError("PSM field %s does not fit float64 exactly" % f)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def cpu_identify(cfg, prots, mods, sp, sample, threads):
     """The oracle (CPU port of the reference's algorithm) on the first `sample` spectra; returns (spectra/s, pairs/s, psms, n)."""
     sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -191,6 +221,8 @@ def run_reference(args, cfg, rank, world):
         pairs += st["n_targets"] + st["n_decoys"]
     dt = time.time() - t0
     e.close()
+    if args.dump_outputs:
+        dump_outputs(psms, args.dump_outputs)
     v = sample * args.steps / dt
     line = {"impl": "reference", "metric": "spectra_per_sec", "value": v, "unit": "spectra/s", "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -284,7 +316,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--c4-spectra", type=int, default=-1, help="size of the strong-scaling set (default 100000 with --config c2, else 0 = skip)")
     ap.add_argument("--no-c4", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the PSM table of the last timed step as DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     cfg = dict(CONFIGS[args.config])
     if args.decoys >= 0:
@@ -442,6 +477,8 @@ def main():
     last = (tick[0] - 1) & 1
     table_all = (psm_alls[last] if world > 1 else psm_devs[last]).cpu().numpy().view(_abi.PSM_DTYPE).reshape(-1, TOP_K)
     crc_all = psm_crc(table_all)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(table_all, args.dump_outputs)
     table_own = psm_devs[last].cpu().numpy().view(_abi.PSM_DTYPE).reshape(-1, TOP_K).copy()
 
     with torch.cuda.stream(ext):
@@ -474,7 +511,7 @@ def main():
         with torch.cuda.stream(ext):
             c4_pass()
             barrier()
-            ms_c4, c4_steps, c4_st = 0.0, 2, None
+            ms_c4, c4_steps, c4_st = 0.0, args.steps, None
             for _ in range(c4_steps):
                 flush.fill_(1)
                 barrier()
