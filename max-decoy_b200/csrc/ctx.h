@@ -72,7 +72,8 @@ struct IdentifyWorkspace {
   DevBuf<uint8_t> cub_tmp;
   // per-call temporaries kept between calls (cudaMalloc/cudaFree inside a call would serialise the device)
   DevBuf<uint64_t> t_size; DevBuf<int16_t> t_K; DevBuf<uint32_t> t_flag, t_pos; DevBuf<int> t_ovf, t_unsorted;
-  DevBuf<uint32_t> t_list, t_off, t_base, t_queue, t_spill, t_blk;
+  DevBuf<uint32_t> t_list, t_off, t_base, t_queue, t_blk;
+  DevBuf<uint4> t_grown; DevBuf<uint8_t> t_route; DevBuf<uint32_t> t_narrow, t_wide;   // decoy rounds: grown attempts (32 B each), repair-pass flags and lists
   DevBuf<md_precursor> t_win;        // MD_VARMOD_EXPANDED: shifted windows, one per (spectrum, count vector)
   // exhaustive mode
   DevBuf<int32_t> ex_comp; DevBuf<uint64_t> ex_cum; DevBuf<uint32_t> ex_ncomp;

@@ -113,6 +113,21 @@ __device__ __forceinline__ uint32_t find_entry(const uint32_t* __restrict__ att_
   return lo;
 }
 
+// One Philox4x32-10 block of the decoy stream (Philox4::refill with c3 = MD_TAG_RANDOM).  Each product is one mul.wide.u32:
+// written as a 64-bit C++ multiply, the compiler added a zero high word (VIADD ..., URZ) behind every IMAD.WIDE.U32.
+__device__ __forceinline__ uint4 philox_block(uint32_t a, uint32_t b, uint32_t c, uint32_t x, uint32_t y) {
+  uint32_t d = MD_TAG_RANDOM;
+#pragma unroll
+  for (int r = 0; r < 10; r++) {
+    uint32_t lo0, hi0, lo1, hi1;
+    asm("{ .reg .b64 t; mul.wide.u32 t, %2, %3; mov.b64 {%0, %1}, t; }" : "=r"(lo0), "=r"(hi0) : "r"(a), "n"(0xD2511F53u));
+    asm("{ .reg .b64 t; mul.wide.u32 t, %2, %3; mov.b64 {%0, %1}, t; }" : "=r"(lo1), "=r"(hi1) : "r"(c), "n"(0xCD9E8D57u));
+    a = hi1 ^ b ^ x; b = lo1; c = hi0 ^ d ^ y; d = lo0;
+    x += 0x9E3779B9u; y += 0xBB67AE85u;
+  }
+  return make_uint4(a, b, c, d);
+}
+
 // Philox4x32-10 output stream of one attempt, buffered in a per-lane shared-memory ring so that the block function runs
 // for the whole warp at once (every kRngPeriod steps of the kernel loop) instead of as a divergent tail behind whichever
 // lane happens to run dry.  The stream is exactly Philox4::next()'s: blocks c0 = 0, 1, 2, ... in order, four words each.
@@ -124,22 +139,17 @@ struct RngRing {
   uint32_t addr;                 // shared-memory address of the lane's kRing words, stride kThreads (accessed through volatile asm only)
   uint32_t k0, k1, c0, c1, c2;   // key, next block, attempt, spectrum
   uint32_t head, count;
-  __device__ __forceinline__ void start(uint64_t seed, uint32_t spectrum_id, uint32_t attempt) {
-    k0 = (uint32_t)seed; k1 = (uint32_t)(seed >> 32); c0 = 0; c1 = attempt; c2 = spectrum_id; head = 0; count = 0;
+  // continue the stream of (seed, spectrum_id, attempt) at word w: block w / 4, its first w % 4 words skipped
+  __device__ __forceinline__ void resume(uint64_t seed, uint32_t spectrum_id, uint32_t attempt, uint32_t w) {
+    k0 = (uint32_t)seed; k1 = (uint32_t)(seed >> 32); c0 = w >> 2; c1 = attempt; c2 = spectrum_id; head = 0; count = 0;
+    produce();
+    head = w & 3u; count = 4u - (w & 3u);
   }
   __device__ __forceinline__ void put(uint32_t t, uint32_t v) const { asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr + (t & (kRing - 1)) * (kThreads * 4u)), "r"(v)); }
   __device__ __forceinline__ void produce() {   // one block -> 4 words into the ring (needs count <= kRing - 4)
-    uint32_t a = c0, b = c1, c = c2, d = MD_TAG_RANDOM, x = k0, y = k1;
-#pragma unroll
-    for (int r = 0; r < 10; r++) {
-      const uint64_t p0 = (uint64_t)0xD2511F53u * a, p1 = (uint64_t)0xCD9E8D57u * c;
-      const uint32_t n0 = (uint32_t)(p1 >> 32) ^ b ^ x, n1 = (uint32_t)p1;
-      const uint32_t n2 = (uint32_t)(p0 >> 32) ^ d ^ y, n3 = (uint32_t)p0;
-      a = n0; b = n1; c = n2; d = n3;
-      x += 0x9E3779B9u; y += 0xBB67AE85u;
-    }
+    const uint4 o = philox_block(c0, c1, c2, k0, k1);
     const uint32_t t = head + count;
-    put(t + 0, a); put(t + 1, b); put(t + 2, c); put(t + 3, d);
+    put(t + 0, o.x); put(t + 1, o.y); put(t + 2, o.z); put(t + 3, o.w);
     c0++; count += 4;
   }
   __device__ __forceinline__ uint32_t next() {
@@ -148,14 +158,13 @@ struct RngRing {
     head++; count--;
     return v;
   }
-  __device__ __forceinline__ uint32_t below(uint32_t n) { return (uint32_t)(((uint64_t)next() * n) >> 32); }
 };
 #ifndef MD_RNG_PERIOD
 #define MD_RNG_PERIOD 8
 #endif
 constexpr uint32_t kRngPeriod = MD_RNG_PERIOD;
 #ifndef MD_REFILL_MIN
-#define MD_REFILL_MIN 8
+#define MD_REFILL_MIN 6
 #endif
 constexpr int kRefillMin = MD_REFILL_MIN;   // free lanes of a warp that trigger a refill
 
@@ -242,29 +251,96 @@ template <uint32_t OFF> __device__ __forceinline__ uint32_t tab_u8(uint32_t addr
   uint32_t v; asm("ld.shared.u8 %0, [%1+%2];" : "=r"(v) : "r"(addr), "n"(OFF)); return v;
 }
 
-struct RandomArgs {
+struct RandomArgs {   // the work items of a round: list entries (spectrum, attempt ordinals) and their prefix of attempt counts
   const md_precursor* prec; const uint32_t* list; const uint32_t* att_off; const uint32_t* att_base;
   const uint32_t* att_blk;              // coarse index into att_off (find_entry_coarse)
   uint32_t n_list, total;
-  uint32_t* queue;                       // work counter of this launch
-  const uint32_t* remap; const uint32_t* remap_n;   // wide pass: work item -> attempt (the narrow pass's spill list), or NULL
-  uint32_t* spill; uint32_t* spill_n;    // narrow pass: attempts that grew past 32 residues, left to the wide pass
   uint64_t seed; int* overflow;
 };
 
+// A grown attempt, from k_decoy_grow to k_decoy_random and k_decoy_finish: its residual d = weight - precursor and the
+// window [dlo, dlo + span] in 32-bit residual space, its length, its RNG counter and the precursor mass.  The alphabet-index
+// sequence is in the attempt's row of AttemptOut::rows.  k_decoy_random writes the final residual of a hit back into d.
+struct __align__(16) GrownAttempt {
+  int32_t d, dlo; uint32_t span, L;
+  uint32_t spectrum_id, attempt; int64_t P;
+};
+
+// Grow phase of REFERENCE_RANDOM (decoy_generator.rs:142-159), one thread per work item of the round: uniform letters until the
+// weight exceeds the upper limit.  A sequence longer than 60 residues (VARCHAR(60) would reject it) is a failure (len = 0) here;
+// every other attempt is flagged for the repair pass of its length -- 32-bit position masks up to `narrow_max` residues, 64-bit
+// ones above -- and k_decoy_random continues its RNG stream at word L.  The sequence goes to the row as alphabet indices in
+// 16-byte stores (the finished words of a chunk wait in registers), not byte by byte.
+constexpr int kGrowThreads = 256;
+__global__ void __launch_bounds__(kGrowThreads) k_decoy_grow(const RandomArgs A, const __grid_constant__ DecoyTables T, AttemptOut O,
+                                                             GrownAttempt* __restrict__ grown, uint8_t* __restrict__ to_narrow,
+                                                             uint8_t* __restrict__ to_wide, uint32_t narrow_max) {
+  __shared__ int32_t s_m[32];
+  if (threadIdx.x < 32) s_m[threadIdx.x] = (int32_t)T.mprime[threadIdx.x];
+  __syncthreads();
+  const uint32_t wi = blockIdx.x * blockDim.x + threadIdx.x;
+  if (wi >= A.total) return;
+  const uint32_t li = find_entry_coarse(A.att_off, A.att_blk, wi);
+  const md_precursor pr = A.prec[A.list[li]];
+  const uint32_t attempt = A.att_base[li] + (wi - A.att_off[li]);
+  uint4* row = reinterpret_cast<uint4*>(O.rows + (size_t)wi * MD_DECOY_ROW);
+  int64_t w = MD_WATER_UDA;
+  uint32_t L = 0, b = 0, word = 0;
+  uint32_t w0 = 0, w1 = 0, w2 = 0;   // the finished words of the current 16-byte chunk, the newest in w2
+  bool dead = false;
+  for (;; b++) {   // Philox block b = words 4b .. 4b+3 = residues 4b .. 4b+3 = the b-th 32-bit word of the row
+    const uint4 r = philox_block(b, attempt, pr.spectrum_id, (uint32_t)A.seed, (uint32_t)(A.seed >> 32));
+    const uint32_t rw[4] = {r.x, r.y, r.z, r.w};
+    bool done = false;
+    word = 0;
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+      if (!done) {
+        const uint32_t a = (uint32_t)(((uint64_t)rw[j] * MD_ALPHABET_SIZE) >> 32);
+        if (L >= MD_MAX_PEPTIDE_LEN) { dead = true; done = true; }
+        else {
+          word |= a << (8 * j); L++;
+          w += s_m[a];
+          done = w > pr.hi;
+        }
+      }
+    }
+    if (done) break;
+    if ((b & 3u) == 3u) row[b >> 2] = make_uint4(w0, w1, w2, word);
+    else { w0 = w1; w1 = w2; w2 = word; }
+  }
+  const int64_t dd = w - pr.mass, dl = pr.lo - pr.mass, sp = pr.hi - pr.lo;
+  if (!dead && (dd > 0x3FFFFFFF || dd < -0x3FFFFFFF || dl > 0x3FFFFFFF || dl < -0x3FFFFFFF || sp < 0 || sp > 0x7FFFFFFF)) { atomicMax(A.overflow, 2); dead = true; }
+  to_narrow[wi] = !dead && L <= narrow_max;
+  to_wide[wi] = !dead && L > narrow_max;
+  if (dead) { O.len[wi] = 0; return; }
+  for (uint32_t k = b & 3u; k < 3u; k++) { w0 = w1; w1 = w2; w2 = word; word = 0; }   // the last chunk: its words in front
+  row[b >> 2] = make_uint4(w0, w1, w2, word);
+  grown[wi] = GrownAttempt{(int32_t)dd, (int32_t)dl, (uint32_t)sp, L, pr.spectrum_id, attempt, pr.mass};
+}
+
+struct RepairArgs {
+  const uint32_t* items; const uint32_t* n_items;   // the attempts of this pass (k_decoy_grow's narrow or wide list) and their count
+  uint32_t* queue;                                   // work counter of this launch
+  GrownAttempt* grown;
+  uint64_t seed; int* overflow;
+};
+
+// Repair phase (modified_peptide.rs:451-508) of the attempts k_decoy_grow left to one pass.
 // One lane = one attempt at a time, run as a flat state machine: every pass of the kernel loop does ONE step for every
 // lane that has an attempt -- the first improving substitution at or behind the pass position, or, when the pass is
 // over, the random kick -- and both kinds of step end in the same "put letter c at position p" code, so the lanes of a
 // warp stay together although their attempts are at different tries / positions / lengths (nested try/position loops
 // would make 31 finished lanes wait for the one that runs all 100 tries).  Lanes whose attempt ends (hit, or 100 tries
-// without one) park until a quarter of the warp is free, then fetch and grow new attempts together.  Inside the loop an
-// attempt is its residual d = weight - precursor in 32 bits (|d| stays far below 2^30 uDa after the grow phase; checked,
-// reported via `overflow`) and the window is [dlo, dlo + span] in the same space.
+// without one) park until kRefillMin lanes of the warp are free, then write their results and load new grown attempts
+// together.  Inside the loop an attempt is its residual d = weight - precursor in 32 bits (|d| stays far below 2^30 uDa
+// after the grow phase; checked, reported via `overflow`) and the window is [dlo, dlo + span] in the same space.  A hit
+// leaves its alphabet-index sequence in the row, its mask, its length and its final d; k_decoy_finish does the rest.
 // VMODE: 0 = no variable modification can apply, 1 = one variable letter without a fixed modification (its positions are
 // tracked, try_variable_modifications needs no walk over the sequence), 2 = anything else (generic enumeration).
 template <int VMODE, class MaskT>
-__global__ void __launch_bounds__(kThreads) k_decoy_random(const RandomArgs A, const __grid_constant__ ModTables M, const __grid_constant__ DecoyTables T,
-                                                           AttemptOut O, PeptideView PV) {
+__global__ void __launch_bounds__(kThreads, sizeof(MaskT) == 4 ? (VMODE < 2 ? 10 : 8) : 1) k_decoy_random(const RepairArgs A, const __grid_constant__ ModTables M, const __grid_constant__ DecoyTables T,
+                                                           AttemptOut O) {
   using MO = MaskOps<MaskT>;
   constexpr uint32_t kBits = MO::bits;
   constexpr bool kNarrow = kBits < MD_MAX_PEPTIDE_LEN;
@@ -297,7 +373,7 @@ __global__ void __launch_bounds__(kThreads) k_decoy_random(const RandomArgs A, c
   const int32_t nn_lo = T.nn_lo, nn_hi = T.nn_hi;
   const int va = VMODE == 1 ? md_alpha_of_code((uint32_t)M.var_simple_code) : -1;
   const int32_t vdelta = VMODE == 1 ? (int32_t)M.var[M.var_simple_code] : 0;
-  const uint32_t total = A.remap ? *A.remap_n : A.total;
+  const uint32_t total = *A.n_items;
 
   bool busy = false, drained = false;
   uint32_t pending = 0;           // 1 = hit, 2 = gave up: the result is written when the free lanes refill together
@@ -309,55 +385,67 @@ __global__ void __launch_bounds__(kThreads) k_decoy_random(const RandomArgs A, c
   auto add_letter = [&](uint32_t a, uint32_t i) { const uint32_t ad = pm_a + a * kPmStride; MO::st(ad, MO::ld(ad) | (MaskT)1 << i); present |= 1u << a; };
   auto del_letter = [&](uint32_t a, uint32_t i) { const uint32_t ad = pm_a + a * kPmStride; const MaskT v = MO::ld(ad) & ~((MaskT)1 << i); MO::st(ad, v); if (v == 0) present &= ~(1u << a); };
   uint32_t wi = 0, L = 0, pos = 0, tries = 0, span = 0, flags = 0;
-  int64_t P = 0;
+  int64_t P = 0;                  // (VMODE 2 only: md_try_variable works on weights)
   int32_t d = 0, dlo = 0;
   MaskT mask = 0, vpos = 0, lmask = 0;
-  RngRing rng; rng.start(A.seed, 0, 0);
+  RngRing rng;
   asm volatile("mov.u32 %0, %1;" : "=r"(rng.addr) : "r"((uint32_t)__cvta_generic_to_shared(s_rng) + 4u * threadIdx.x));
 
   uint32_t rng_timer = 1;
   for (;;) {
-    // ---- refill: when at least 8 lanes are free (or nobody works), they fetch and grow new attempts together
+    // ---- refill: when at least kRefillMin lanes are free (or nobody works), they write their results and load new attempts together
     uint32_t busy_m = __ballot_sync(0xffffffffu, busy);
     uint32_t free_m = 0;
     if (__popc(busy_m) <= 32 - kRefillMin) free_m = __ballot_sync(0xffffffffu, !busy && (!drained || pending));
     if (free_m && (__popc(free_m) >= kRefillMin || busy_m == 0)) {
-      if (!busy && pending) { store_attempt(O, wi, seq, pending == 1 ? L : 0, (uint64_t)mask, P + d, T, PV); pending = 0; }
+      if (!busy && pending) {
+        if (pending == 1) {   // the final sequence (alphabet indices) back into the row, 16 bytes at a time
+          uint4* row = reinterpret_cast<uint4*>(O.rows + (size_t)wi * MD_DECOY_ROW);
+#pragma unroll 1
+          for (uint32_t c = 0; 16u * c < L; c++) {
+            uint32_t wd[4];
+#pragma unroll
+            for (uint32_t j = 0; j < 16; j++) {
+              const uint32_t i = 16u * c + j;
+              const uint32_t a = i < L ? seq.get(i) : 0u;
+              wd[j >> 2] = (j & 3) ? wd[j >> 2] | a << (8 * (j & 3)) : a;
+            }
+            row[c] = make_uint4(wd[0], wd[1], wd[2], wd[3]);
+          }
+          O.mask[wi] = (uint64_t)mask; A.grown[wi].d = d;
+        }
+        O.len[wi] = pending == 1 ? (uint8_t)L : 0;
+        pending = 0;
+      }
       if (!busy && !drained) {
         const uint32_t q = atomicAdd(A.queue, 1u);
         if (q >= total) drained = true;
         else {
-          wi = A.remap ? A.remap[q] : q;
-          const uint32_t li = find_entry_coarse(A.att_off, A.att_blk, wi);
-          const md_precursor pr = A.prec[A.list[li]];
-          P = pr.mass;
-          rng.start(A.seed, pr.spectrum_id, A.att_base[li] + (wi - A.att_off[li]));
-          // grow (decoy_generator.rs:142-159): uniform letters until the weight exceeds the upper limit
-          int64_t w = MD_WATER_UDA;
-          L = 0; mask = 0; vpos = 0; present = 0; bool dead = false;
+          wi = A.items[q];
+          const GrownAttempt* g = A.grown + wi;
+          L = g->L; d = g->d; dlo = g->dlo; span = g->span;
+          if (VMODE == 2) P = g->P;
+          rng.resume(A.seed, g->spectrum_id, g->attempt, L);   // the grow phase drew L words
+          // the grown sequence into the lane's shared-memory state: letters, per-letter position masks, variable positions
+          mask = 0; vpos = 0; present = 0;
           for (int a = 0; a < MD_ALPHABET_SIZE; a++) MO::st(pm_a + a * kPmStride, (MaskT)0);
-          for (;;) {
-            const uint32_t a = rng.below(MD_ALPHABET_SIZE);
-            if (L >= MD_MAX_PEPTIDE_LEN) { dead = true; break; }  // > 60 residues: VARCHAR(60) would reject it
-            if (!kNarrow || L < kBits) {
-              if (VMODE == 1 && (int)a == va) vpos |= (MaskT)1 << L;
-              add_letter(a, L); seq.set(L, a);
-            }
-            L++;
-            w += (int32_t)tab_u32<tabs::mprime>(tb + 4u * a);
-            if (w > pr.hi) break;
-          }
-          if (kNarrow && !dead && L > kBits) {
-            A.spill[atomicAdd(A.spill_n, 1u)] = wi;       // the wide pass runs this attempt (same RNG stream, same slot)
-          } else {
-            const int64_t dd = w - P, dl = pr.lo - P, sp = pr.hi - pr.lo;
-            if (!dead && (dd > 0x3FFFFFFF || dd < -0x3FFFFFFF || dl > 0x3FFFFFFF || dl < -0x3FFFFFFF || sp < 0 || sp > 0x7FFFFFFF)) { flags |= 2u; dead = true; }
-            if (dead) store_attempt(O, wi, seq, 0, 0, 0, T, PV);
-            else {
-              busy = true; tries = 0; pos = 0; d = (int32_t)dd; dlo = (int32_t)dl; span = (uint32_t)sp;
-              lmask = L >= kBits ? ~(MaskT)0 : (((MaskT)1 << L) - 1);
+          const uint4* row = reinterpret_cast<const uint4*>(O.rows + (size_t)wi * MD_DECOY_ROW);
+#pragma unroll 1
+          for (uint32_t c = 0; 16u * c < L; c++) {
+            const uint4 v = row[c];
+            const uint32_t wd[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+            for (uint32_t j = 0; j < 16; j++) {
+              const uint32_t i = 16u * c + j;
+              if (i < L) {
+                const uint32_t a = (wd[j >> 2] >> (8 * (j & 3))) & 0xFFu;
+                if (VMODE == 1 && (int)a == va) vpos |= (MaskT)1 << i;
+                add_letter(a, i); seq.set(i, a);
+              }
             }
           }
+          busy = true; tries = 0; pos = 0;
+          lmask = L >= kBits ? ~(MaskT)0 : (((MaskT)1 << L) - 1);
         }
       }
       busy_m = __ballot_sync(0xffffffffu, busy);
@@ -455,6 +543,46 @@ __global__ void __launch_bounds__(kThreads) k_decoy_random(const RandomArgs A, c
     }
   }
   if (flags) atomicMax(A.overflow, (flags & 4u) ? 3 : 2);
+}
+
+// Finish phase, one thread per work item of the round: every hit k_decoy_random left (alphabet indices in the row, final d in
+// GrownAttempt) becomes what store_attempt writes -- residue codes padded with MD_CODE_OTHER to the whole row, the sequence
+// hash, the weight P + d -- unless it is a peptide of the index (len = 0).
+__global__ void __launch_bounds__(256) k_decoy_finish(uint32_t total, const __grid_constant__ DecoyTables T, AttemptOut O,
+                                                      const GrownAttempt* __restrict__ grown, PeptideView PV) {
+  __shared__ uint8_t s_code[32];
+  if (threadIdx.x < 32) s_code[threadIdx.x] = T.code_of_a[threadIdx.x];
+  __syncthreads();
+  const uint32_t wi = blockIdx.x * blockDim.x + threadIdx.x;
+  if (wi >= total) return;
+  const uint32_t L = O.len[wi];
+  if (L == 0) return;
+  uint8_t* rowb = O.rows + (size_t)wi * MD_DECOY_ROW;
+  uint4* row = reinterpret_cast<uint4*>(rowb);
+  const uint32_t pad = MD_CODE_OTHER * 0x01010101u;
+  uint64_t h = md_hash_init();
+#pragma unroll
+  for (uint32_t c = 0; c < MD_DECOY_ROW / 16; c++) {
+    uint32_t wd[4] = {pad, pad, pad, pad};
+    if (16u * c < L) {
+      const uint4 v = row[c];
+      const uint32_t in[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (uint32_t j = 0; j < 16; j++) {
+        const uint32_t i = 16u * c + j;
+        if (i < L) {
+          const uint32_t code = s_code[(in[j >> 2] >> (8 * (j & 3))) & 0xFFu];
+          h = md_hash_step(h, md_letter_of(code));
+          wd[j >> 2] = (wd[j >> 2] & ~(0xFFu << (8 * (j & 3)))) | code << (8 * (j & 3));
+        }
+      }
+    }
+    row[c] = make_uint4(wd[0], wd[1], wd[2], wd[3]);
+  }
+  h = md_hash_fin(h, L);
+  if (is_peptide([rowb](uint32_t i) { return md_letter_of(rowb[i]); }, L, h, PV.ht_key, PV.ht_val, PV.ht_mask, PV.seq, PV.off, PV.len)) { O.len[wi] = 0; return; }
+  const GrownAttempt& g = grown[wi];
+  O.w[wi] = g.P + g.d; O.hash[wi] = h;
 }
 
 // Terminal modifications (position N / C): the attempt restated literally, one lane per attempt -- the weight of a residue
@@ -777,10 +905,10 @@ __global__ void __launch_bounds__(256) k_decoy_select_n2(const uint32_t* __restr
 }
 
 template <class MaskT>
-void launch_random(md_ctx* ctx, int vmode, uint32_t grid, const RandomArgs& RA, const DecoyTables& T, const AttemptOut& O, const PeptideView& PV) {
-  if (vmode == 0) MD_LAUNCH(ctx, (k_decoy_random<0, MaskT>), grid, kThreads, 0, RA, ctx->mods, T, O, PV);
-  else if (vmode == 1) MD_LAUNCH(ctx, (k_decoy_random<1, MaskT>), grid, kThreads, 0, RA, ctx->mods, T, O, PV);
-  else MD_LAUNCH(ctx, (k_decoy_random<2, MaskT>), grid, kThreads, 0, RA, ctx->mods, T, O, PV);
+void launch_random(md_ctx* ctx, int vmode, uint32_t grid, const RepairArgs& RA, const DecoyTables& T, const AttemptOut& O) {
+  if (vmode == 0) MD_LAUNCH(ctx, (k_decoy_random<0, MaskT>), grid, kThreads, 0, RA, ctx->mods, T, O);
+  else if (vmode == 1) MD_LAUNCH(ctx, (k_decoy_random<1, MaskT>), grid, kThreads, 0, RA, ctx->mods, T, O);
+  else MD_LAUNCH(ctx, (k_decoy_random<2, MaskT>), grid, kThreads, 0, RA, ctx->mods, T, O);
 }
 template <class MaskT>
 int random_occupancy(int vmode) {
@@ -1001,9 +1129,6 @@ void decoys_generate_dev(md_ctx* ctx, uint32_t n, uint32_t n_per, int mode, uint
     MD_CUDA(cudaMemcpyAsync(d_base.p, base.data(), n_list * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
     MD_CUDA(cudaEventRecord(ctx->ev[4], ctx->stream));
     if (mode == MD_DECOY_REFERENCE_RANDOM) {
-      // narrow pass (32-bit position masks) over every attempt, then the wide pass over those that grew past 32 residues
-      MD_CUDA(cudaMemsetAsync(d_queue.p, 0, 4 * sizeof(uint32_t), ctx->stream));
-      W.t_spill.need((size_t)total + 1);
       RandomArgs RA;
       {   // coarse index: entry of every 1024th work item (+ one past the end)
         const uint32_t nb = (total >> kBlkLog) + 2;
@@ -1020,16 +1145,24 @@ void decoys_generate_dev(md_ctx* ctx, uint32_t n, uint32_t n_per, int mode, uint
       RA.prec = W.prec.p; RA.list = d_list.p; RA.att_off = d_off.p; RA.att_base = d_base.p; RA.n_list = n_list; RA.total = total; RA.att_blk = W.t_blk.p;
       RA.seed = seed; RA.overflow = d_ovf.p;
       if (ctx->mods.has_terminal) {
-        RA.queue = d_queue.p; RA.remap = nullptr; RA.remap_n = nullptr; RA.spill = nullptr; RA.spill_n = nullptr;
         MD_LAUNCH(ctx, k_decoy_random_terminal, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * 8u), kThreads, 0, RA, ctx->mods, T, O, PV);
-      } else if (!wide_only) {
-        RA.queue = d_queue.p; RA.remap = nullptr; RA.remap_n = nullptr; RA.spill = W.t_spill.p; RA.spill_n = d_queue.p + 1;
-        launch_random<uint32_t>(ctx, vmode, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * (uint32_t)occ_narrow), RA, T, O, PV);
-        RA.queue = d_queue.p + 2; RA.remap = W.t_spill.p; RA.remap_n = d_queue.p + 1; RA.spill = nullptr; RA.spill_n = nullptr;
-        launch_random<uint64_t>(ctx, vmode, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * (uint32_t)occ_wide), RA, T, O, PV);
       } else {
-        RA.queue = d_queue.p; RA.remap = nullptr; RA.remap_n = nullptr; RA.spill = nullptr; RA.spill_n = nullptr;
-        launch_random<uint64_t>(ctx, vmode, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * (uint32_t)occ_wide), RA, T, O, PV);
+        // grow every attempt; repair those up to 32 residues with 32-bit position masks, then the longer ones with 64-bit
+        // masks; finish the hits.  The two lists keep the work-item order (spectra by mass: neighbouring lanes repair
+        // sequences of similar length).
+        const size_t tpad = ((size_t)total + 15) & ~(size_t)15;
+        W.t_grown.need(2 * (size_t)total + 2); W.t_route.need(2 * tpad); W.t_narrow.need((size_t)total + 1); W.t_wide.need((size_t)total + 1);
+        GrownAttempt* grown = reinterpret_cast<GrownAttempt*>(W.t_grown.p);
+        uint8_t* to_narrow = W.t_route.p; uint8_t* to_wide = W.t_route.p + tpad;
+        MD_CUDA(cudaMemsetAsync(d_queue.p, 0, 4 * sizeof(uint32_t), ctx->stream));
+        MD_LAUNCH(ctx, k_decoy_grow, blocks(total, kGrowThreads), kGrowThreads, 0, RA, T, O, grown, to_narrow, to_wide, wide_only ? 0u : 32u);
+        cubx_select_flagged_index(ctx, to_narrow, W.t_narrow.p, d_queue.p + 1, total);
+        cubx_select_flagged_index(ctx, to_wide, W.t_wide.p, d_queue.p + 3, total);
+        RepairArgs R{W.t_narrow.p, d_queue.p + 1, d_queue.p, grown, seed, d_ovf.p};
+        if (!wide_only) launch_random<uint32_t>(ctx, vmode, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * (uint32_t)occ_narrow), R, T, O);
+        R = RepairArgs{W.t_wide.p, d_queue.p + 3, d_queue.p + 2, grown, seed, d_ovf.p};
+        launch_random<uint64_t>(ctx, vmode, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * (uint32_t)occ_wide), R, T, O);
+        MD_LAUNCH(ctx, k_decoy_finish, blocks(total, 256), 256, 0, total, T, O, grown, PV);
       }
     } else {
       MD_LAUNCH(ctx, k_decoy_permute, blocks(total, kThreads), kThreads, 0, W.prec.p, d_list.p, d_off.p, d_base.p, n_list, total, seed, T, W.cand_off.p,
