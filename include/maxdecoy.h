@@ -205,7 +205,10 @@ MD_API void md_candidate_table_free(md_candidate_table* t);
 typedef enum md_decoy_mode {
   /* DecoyGenerator::generate_decoys + swap_amino_acids_to_hit_mass_tolerance
    * (utility/decoy_generator.rs:127-188; modified_peptide.rs:451-508) with a counter-based
-   * RNG keyed by (seed, spectrum_id, attempt); the reference's RNG is unseeded. */
+   * RNG keyed by (seed, spectrum_id, attempt); the reference's RNG is unseeded.  The repair loop works in 32-bit
+   * residuals: md_generate_decoys returns MD_ERR_UNSUPPORTED when a residue with its fixed modification (or a variable
+   * modification) reaches 2^29 uDa (536.87 Da), or when a precursor window reaches further than 2^30 - 1 uDa
+   * (1073.74 Da) from its mass; the reference has neither limit. */
   MD_DECOY_REFERENCE_RANDOM = 0,
   /* every sequence whose fixed-modification weight lies in the window: compositions (count vectors over MD_ALPHABET)
    * in ascending lexicographic order, per composition its distinct permutations in ascending lexicographic order;

@@ -20,7 +20,16 @@ namespace {
 inline uint32_t blocks(uint64_t n, uint32_t bs = 256) { return (uint32_t)((n + bs - 1) / bs); }
 
 constexpr int kThreads = 128;          // lanes per CTA of the attempt kernels
-constexpr int kMaxRoundAttempts = 4096;  // per list entry (bounds the selection kernel's shared memory)
+// MD_ROUND_ATTEMPTS and MD_SELECT_SMEM_MAX (test builds only) shrink the list entries and the hash selection's shared-memory
+// budget, so that small inputs run several levels per round and reach k_decoy_select_n2
+#ifndef MD_ROUND_ATTEMPTS
+#define MD_ROUND_ATTEMPTS 4096
+#endif
+#ifndef MD_SELECT_SMEM_MAX
+#define MD_SELECT_SMEM_MAX (220 * 1024)
+#endif
+constexpr int kMaxRoundAttempts = MD_ROUND_ATTEMPTS;  // per list entry (bounds the selection kernel's shared memory)
+static_assert(kMaxRoundAttempts >= 1 && kMaxRoundAttempts <= 8192, "k_decoy_select keeps one thread's share of an entry in a 32-bit mask");
 constexpr int kRoundLevels = 4;          // list entries one spectrum can have in a round: its attempts in consecutive chunks, selected one after the other
 
 // letter tables in alphabet-index space, built once per call on the host
@@ -1178,7 +1187,9 @@ void decoys_generate_dev(md_ctx* ctx, uint32_t n, uint32_t n_per, int mode, uint
       uint32_t slots = 1024; while ((uint64_t)slots * 3 < (uint64_t)need * 4) slots <<= 1;   // load factor <= 0.75 even if every attempt succeeded
       max_na = (max_na + 7u) & ~7u;
       const size_t smem = (size_t)slots * 12 + (size_t)max_na * 10;
-      if (smem <= 220 * 1024) {
+      const bool hashed = smem <= (size_t)(MD_SELECT_SMEM_MAX);
+      if (ctx->trace) fprintf(stderr, "[md_trace]   decoy select round %d level %d: entries=%u kernel=%s\n", round, c, le - lb, hashed ? "hash" : "n2");
+      if (hashed) {
         MD_CUDA(cudaFuncSetAttribute(k_decoy_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         MD_LAUNCH(ctx, k_decoy_select, le - lb, 256, smem, d_list.p + lb, d_off.p + lb, d_base.p + lb, n_per, slots, max_na, O, (uint64_t)n * n_per, W.dec_rows.p, W.dec_len.p, W.dec_mask.p,
                   W.dec_w.p, W.dec_hash.p, W.dec_attempt.p, W.dec_count.p);

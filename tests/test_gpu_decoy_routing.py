@@ -5,13 +5,13 @@ import numpy as np
 import pytest
 
 import maxdecoy
-from maxdecoy import synth
+from maxdecoy import Modification, synth
 from oracle_lib import oracle_engine
 import workloads as wl
 
 pytestmark = pytest.mark.gpu
 
-MASSES = (3_550_000_000, 3_700_000_000, 3_850_000_000, 6_700_000_000, 6_900_000_000, 7_050_000_000)
+PHOSPHO_S = Modification("x:21", "Phospho", "A", False, "S", 79.966331)
 
 
 @pytest.fixture(scope="module")
@@ -28,13 +28,14 @@ def cpu():
     e.close()
 
 
-@pytest.mark.parametrize("mods,nvar", [((synth.CAM,), 0), ((synth.CAM, synth.OXM), 3)])
+@pytest.mark.parametrize("mods,nvar", [((synth.CAM,), 0), ((synth.CAM, synth.OXM), 3), ((synth.CAM, synth.OXM, PHOSPHO_S), 2)])
 def test_decoy_lengths_at_routing_edges_bit_exact(gpu, cpu, mods, nvar, monkeypatch):
+    """No variable letter, one (the position-mask path) and two (the generic enumeration)."""
     for e in (gpu, cpu):
         e.digest(list(wl.proteins(300)), 2, 5, 50)
         e.set_modifications(list(mods), nvar)
         e.index_build()
-    pre = [(m, m - m // 100_000, m + m // 100_000, 2 + i % 3, 900 + i) for i, m in enumerate(MASSES)]
+    pre = wl.routing_precursors()
     dc = cpu.generate_decoys(pre, 60, maxdecoy.DECOY_REFERENCE_RANDOM, seed=5)
     dg = gpu.generate_decoys(pre, 60, maxdecoy.DECOY_REFERENCE_RANDOM, seed=5)
     for k in dc:

@@ -110,10 +110,7 @@ def test_decoys_random_long_sequences_bit_exact(gpu, cpu, mods, nvar, monkeypatc
     one; sequences near the 60-residue cap are dropped.  Also: the 64-bit pass alone gives the same decoys."""
     for e in (gpu, cpu):
         _setup(e, 300, 2, mods, nvar)
-    pre = []
-    for i, m in enumerate((1_700_800_000, 2_900_400_000, 3_600_700_000, 4_300_100_000, 5_200_900_000, 6_400_300_000)):
-        tol = m // 100_000
-        pre.append((m, m - tol, m + tol, 2 + i % 3, 500 + i))
+    pre = wl.heavy_precursors()
     dc = cpu.generate_decoys(pre, 120, maxdecoy.DECOY_REFERENCE_RANDOM, seed=3)
     dg = gpu.generate_decoys(pre, 120, maxdecoy.DECOY_REFERENCE_RANDOM, seed=3)
     assert_tables_equal(dg, dc)
@@ -125,18 +122,11 @@ def test_decoys_random_long_sequences_bit_exact(gpu, cpu, mods, nvar, monkeypatc
 
 
 def test_decoys_random_degenerate_masses_bit_exact(gpu, cpu):
-    """Modification sets that make letters collide: G+14.01565 equals A to the micro-dalton (an equal-mass run: ties go to
-    the lower alphabet index), S+12.03637 lands 10 uDa under V and T+27.04728 lands 1 uDa above K (near-ties on either side of
-    a midpoint), plus two variable letters, one of them also fixed (the generic variable-modification path).  The
+    """The modification sets of workloads.degenerate_mod_sets make letters collide (equal masses, near-ties on either side
+    of a midpoint) and add two variable letters, one of them also fixed (the generic variable-modification path).  The
     substitution search of the kernel (bucket tables) must agree with the oracle's literal 20-way scan."""
-    from maxdecoy import Modification
-    fix_g = Modification("x:1", "GtoA", "A", True, "G", 14.015650)
-    fix_s = Modification("x:2", "StoV", "A", True, "S", 12.036370)
-    fix_t = Modification("x:3", "TtoK", "A", True, "T", 27.047280)
-    var_m = Modification("unimod:35", "Oxidation", "A", False, "M", 15.994915)
-    var_g = Modification("x:4", "Gvar", "A", False, "G", 0.984016)
     sp, _ = wl.spectra(300, 16, 2)
-    for mods, nvar in (((synth.CAM, fix_g, fix_s, fix_t), 0), ((synth.CAM, fix_g, fix_s, var_m, var_g), 2)):
+    for mods, nvar in wl.degenerate_mod_sets():
         for e in (gpu, cpu):
             _setup(e, 300, 2, mods, nvar)
         pre = wl.precursors_of(cpu, sp)
@@ -436,23 +426,12 @@ def test_gather_psms_single_rank_and_device_pointers(gpu):
     gpu.comm_destroy()
 
 
-def test_decoy_selection_is_exact_when_hashes_collide(cpu, tmp_path):
+def test_decoy_selection_is_exact_when_hashes_collide(cpu):
     """k_decoy_select finds duplicates through a hash set; a success whose hash is already carried by a different sequence
     must still be kept.  A test build of the library that keeps only 6 bits of the hashes makes such collisions the rule:
     its decoys must still equal the oracle's (which compares strings)."""
-    import os
-    import shutil
-    import subprocess
-    csrc = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "max-decoy_b200", "csrc")
-    if shutil.which("nvcc") is None and not os.path.exists("/usr/local/cuda/bin/nvcc"):
-        pytest.skip("no nvcc to make the test build")
-    nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
-    obj, so = str(tmp_path / "decoy_hash6.o"), str(tmp_path / "libmaxdecoy_hash6.so")
-    flags = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-Xcompiler", "-fPIC,-fvisibility=hidden", "--expt-relaxed-constexpr", "-cudart", "static"]
-    subprocess.check_call([nvcc] + flags + ["-DMD_SELECT_HASH_MASK=0x3Full", "-c", os.path.join(csrc, "decoy.cu"), "-o", obj])
-    others = [os.path.join(csrc, f) for f in ("api.o", "comm.o", "digest.o", "index.o", "exhaustive.o", "score.o")]
-    subprocess.check_call([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-cudart", "static", "-o", so, obj] + others + ["-ldl"])
-    g = maxdecoy.Engine(lib=maxdecoy.load(so))
+    import testbuild
+    g = testbuild.engine(["-DMD_SELECT_HASH_MASK=0x3Full"])
     try:
         prots = list(wl.proteins(300))
         for e in (g, cpu):

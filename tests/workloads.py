@@ -35,6 +35,31 @@ def precursors_of(engine, sp, lppm=10, uppm=10):
     return out
 
 
+def heavy_precursors():
+    """Heavy precursors (1.7-6.4 kDa, 10 ppm): decoy attempts grow past 32 residues, some past 60."""
+    return [(m, m - m // 100_000, m + m // 100_000, 2 + i % 3, 500 + i)
+            for i, m in enumerate((1_700_800_000, 2_900_400_000, 3_600_700_000, 4_300_100_000, 5_200_900_000, 6_400_300_000))]
+
+
+def routing_precursors():
+    """Precursors whose decoys include sequences of exactly 32, 33 and 60 residues (the repair passes' routing edges)."""
+    return [(m, m - m // 100_000, m + m // 100_000, 2 + i % 3, 900 + i)
+            for i, m in enumerate((3_550_000_000, 3_700_000_000, 3_850_000_000, 6_700_000_000, 6_900_000_000, 7_050_000_000))]
+
+
+def degenerate_mod_sets():
+    """Modification sets that make letters collide: G+14.01565 equals A to the micro-dalton (an equal-mass run: ties go to
+    the lower alphabet index), S+12.03637 lands 10 uDa under V and T+27.04728 lands 1 uDa above K (near-ties on either side of
+    a midpoint), plus two variable letters, one of them also fixed (the generic variable-modification path)."""
+    from maxdecoy import Modification
+    fix_g = Modification("x:1", "GtoA", "A", True, "G", 14.015650)
+    fix_s = Modification("x:2", "StoV", "A", True, "S", 12.036370)
+    fix_t = Modification("x:3", "TtoK", "A", True, "T", 27.047280)
+    var_m = Modification("unimod:35", "Oxidation", "A", False, "M", 15.994915)
+    var_g = Modification("x:4", "Gvar", "A", False, "G", 0.984016)
+    return [((synth.CAM, fix_g, fix_s, fix_t), 0), ((synth.CAM, fix_g, fix_s, var_m, var_g), 2)]
+
+
 def decoy_strings(table):
     raw = table["seq"].tobytes()
     so = table["seq_off"]
