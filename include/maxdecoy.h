@@ -265,7 +265,11 @@ typedef struct md_search_params {
   int64_t upper_ppm;            /* -u */
   int64_t abs_lower_uda;        /* if abs_lower_uda|abs_upper_uda != 0: window = [P-abs_lower, P+abs_upper] (open search) */
   int64_t abs_upper_uda;
-  double fragment_tolerance;    /* --fragmentation-tolerance, Comet fragment_bin_tol (comet_parameter.rs:103) */
+  double fragment_tolerance;    /* --fragmentation-tolerance, Comet fragment_bin_tol (comet_parameter.rs:103); 0.0001..2 Da,
+                                 * rounded to whole uDa (w).  The CUDA library refuses with MD_ERR_UNSUPPORTED (the oracle
+                                 * accepts): a scored spectrum whose table needs more than 2^26 bins, i.e. a usable peak at
+                                 * m/z >= (2^26 - 76) * w (6.71 kDa at 0.0001 Da); a residue whose mass with its fixed and
+                                 * variable modifications reaches 2^22 * w (419 Da at 0.0001 Da). */
   uint32_t n_decoys;            /* -d */
   int32_t decoy_mode;           /* md_decoy_mode */
   uint64_t seed;

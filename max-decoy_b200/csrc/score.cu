@@ -1461,6 +1461,9 @@ void score_run_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const md_
   MD_CUDA(cudaMemcpyAsync(&n_targets, W.cand_off.p + n, sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
   MD_CUDA(cudaStreamSynchronize(ctx->stream));
   MD_REQUIRE(!h_pre[0], MD_ERR_INVALID, "spectra: peaks of a spectrum must be sorted by m/z");
+  // a table beyond kMaxBins is refused on every path: k_build_tables would leave such a spectrum unscored, k_score flags it
+  MD_REQUIRE(h_pre[2] < 0 || (uint64_t)h_pre[2] + kXcorrOffset + 1 <= kMaxBins, MD_ERR_UNSUPPORTED,
+             "a spectrum needs more than 2^26 fragment bins or has more than 2^24 candidates");
   if (want_all) { W.tscore.need(n_targets + 1); W.dscore.need((size_t)n * n_per + 1); }
   // Few spectra with very many candidates each (open searches) would leave SMs idle and make one CTA walk hundreds of
   // chunks: split every spectrum into `parts` work items (contiguous ranges of candidate chunks; each builds the table
