@@ -92,7 +92,7 @@ void identify_batch(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const md
   decoys_generate_dev(ctx, S.n, p.n_decoys, p.decoy_mode, p.seed);
   ctx->mark("decoys");
   MD_CUDA(cudaEventRecord(ctx->ev[2], s));
-  score_run_dev(ctx, S, n_peaks, p, p.n_decoys, psm_dev, want_all);
+  score_run_dev(ctx, S, p, p.n_decoys, psm_dev, want_all);
   MD_CUDA(cudaEventRecord(ctx->ev[3], s));
   MD_CUDA(cudaStreamSynchronize(s));
   ctx->mark("score");

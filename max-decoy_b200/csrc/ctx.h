@@ -67,6 +67,7 @@ struct IdentifyWorkspace {
   DevBuf<int64_t> tscore; DevBuf<int64_t> dscore;
   DevBuf<uint32_t> left_list;        // spectra the pipelined score kernel left to k_score
   DevBuf<uint8_t> tab_pool, tab_desc; DevBuf<uint16_t> cand_order;   // k_build_tables / k_cand_order -> k_score_pipe
+  bool tables_built = false;         // score_prepare_dev built the current batch's table records: score_run_dev may use k_score_pipe
   DevBuf<uint32_t> sched_key, sched_val, sched;                      // the order in which k_score_pipe takes the spectra
   DevBuf<unsigned long long> part_top; DevBuf<uint32_t> parts_done;   // spectra split into parts (open searches): per-part top-k keys, arrival counters
   DevBuf<uint8_t> cub_tmp;
@@ -159,7 +160,7 @@ void decoys_export(md_ctx* ctx, uint32_t n, uint32_t n_per, md_decoy_table* out)
 // bins the n spectra (device SoA), scores targets+decoys, writes PSM rows
 struct SpectraDev { uint32_t n; const double* pmz; const uint8_t* charge; const uint32_t* sid; const uint64_t* peak_off; const double* peak_mz; const float* peak_int; };
 void score_prepare_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const md_search_params& p);
-void score_run_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const md_search_params& p, uint32_t n_per, md_psm* psm_dev, bool want_all);
+void score_run_dev(md_ctx* ctx, const SpectraDev& S, const md_search_params& p, uint32_t n_per, md_psm* psm_dev, bool want_all);
 void precursors_dev(md_ctx* ctx, const SpectraDev& S, const md_search_params& p, uint32_t id_base);
 
 size_t cub_temp_bytes_max(size_t n);

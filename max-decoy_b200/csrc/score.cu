@@ -52,6 +52,7 @@ constexpr uint32_t kPeakCap = 512;         // binned peaks staged in shared memo
 constexpr uint32_t kMaxBins = 1u << 26;    // table bins per spectrum (bins must stay far below kStop)
 constexpr uint32_t kMaxTopK = 128;
 constexpr uint32_t kFastTopK = 8;
+constexpr uint32_t kMaxParts = 16;         // most work items a spectrum is split into (merge_parts)
 
 // ------------------------------------------------------------------------------------------------
 // precursor windows: tasks/identification.rs:203-211 (utility/mod.rs:9-11; models/mass/mod.rs:6-8,14-16)
@@ -201,15 +202,13 @@ struct ScoreArgs {
   uint32_t* work;
   unsigned long long* stat64;  // [0] pairs scored, [1] algorithmic bytes (14 + len per pair)
   int* error;                  // set when a spectrum needs more table bins than kMaxBins
-  unsigned long long* timing;  // MD_SCORE_TIMING=1: per-phase SM cycles summed over CTAs (thread 0's clock), else NULL
   // spectra with very many candidates (open searches) are split into `parts` work items, one contiguous range of candidate
   // chunks each; a part leaves its K best keys in part_top and the last part to finish (parts_done) writes the PSM rows
   uint32_t parts; unsigned long long* part_top; uint32_t* parts_done;
   uint16_t* gmap; uint32_t* gbits; uint32_t gmap_stride;   // per-CTA block map / block bitmap in HBM for tables beyond kMapCap blocks
-  // work items: n_work spectra, work item i = spectrum remap[i] (or i itself without a list).  The pipelined kernel leaves the
-  // spectra it cannot hold in left_list / left_n; k_score then runs over that list.
-  uint32_t n_work; const uint32_t* remap; uint32_t* left_list; uint32_t* left_n;
-  const uint32_t* n_work_dev;   // if set: the number of work items is read from device memory (the list another kernel has just left)
+  // k_score's spectra: n_work of them, spectrum remap[i] (or i itself without a list) -- the whole batch, or the spectra
+  // k_build_tables left to k_score
+  uint32_t n_work; const uint32_t* remap;
 };
 
 __device__ __forceinline__ uint32_t div3(uint32_t x) { return __umulhi(x, 0xAAAAAAABu) >> 1; }
@@ -423,7 +422,6 @@ struct SpecShared {
   unsigned long long top[kMaxTopK];
   unsigned long long wtop[2][kScoreThreads / 32][kFastTopK];  // per-warp best keys of a spectrum, descending
   FinRecord fin[2];         // what the finish warp needs to write that spectrum's PSM rows
-  long long tacc[8];
   uint32_t hist[64];        // candidates per length (counting sort of a chunk by the whole CTA)
   uint32_t unit;            // next unit of the current tile pass
   uint32_t nact;            // occupied table blocks of the spectrum
@@ -441,6 +439,66 @@ __device__ __forceinline__ uint32_t cand_len(const ScoreArgs& A, uint32_t s, uin
   return u < nt ? (uint32_t)(A.cand_desc[t0c + u] >> 40) & 0xFF : A.dec_len[(uint64_t)s * n_per + (u - nt)];
 }
 
+// One warp: the exclusive popcount prefix of the occupied-block bitmap bits[0, nwords) into pre[] (the compressed block of
+// the first occupied block of each word); returns the number of occupied blocks to every lane.
+__device__ __forceinline__ uint32_t warp_bitmap_prefix(const uint32_t* bits, uint32_t* pre, uint32_t nwords) {
+  const uint32_t lane = threadIdx.x & 31;
+  uint32_t run = 0;
+  for (uint32_t base = 0; base < nwords; base += 32) {
+    const uint32_t i = base + lane;
+    const uint32_t c = i < nwords ? (uint32_t)__popc(bits[i]) : 0u;
+    uint32_t incl = c;
+    for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((int)lane >= o) incl += t; }
+    if (i < nwords) pre[i] = run + incl - c;
+    run += __shfl_sync(0xffffffffu, incl, 31);
+  }
+  return run;
+}
+
+// One warp: the 64-bucket length histogram of a counting sort, in place, into its exclusive prefix (each bucket's first slot).
+__device__ __forceinline__ void warp_hist64_prefix(uint32_t* hist) {
+  const uint32_t lane = threadIdx.x & 31;
+  const uint32_t h0 = hist[2 * lane], h1 = hist[2 * lane + 1];
+  uint32_t incl = h0 + h1;
+  for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((int)lane >= o) incl += t; }
+  hist[2 * lane] = incl - h0 - h1; hist[2 * lane + 1] = incl - h1;
+}
+
+// A spectrum split into parts: the work item leaves its K best keys (lane r: its r-th best).  The last part of the spectrum to
+// arrive merges them all (lane r gets the spectrum's r-th best key) and its warp writes the rows; the others get last = false.
+// (The key comes back by value: an out-parameter would keep the caller's key in local memory.)
+struct PartMerge { bool last; unsigned long long best; };
+__device__ __noinline__ PartMerge merge_parts(const ScoreArgs& A, uint32_t s, uint32_t part, uint32_t parts, uint32_t K, unsigned long long best) {
+  const uint32_t lane = threadIdx.x & 31;
+  unsigned long long* pt = A.part_top + (size_t)s * parts * kFastTopK;
+  if (lane < kFastTopK) pt[part * kFastTopK + lane] = lane < K ? best : 0ull;
+  __threadfence();
+  __syncwarp();
+  uint32_t arrived = 0;
+  if (lane == 0) arrived = atomicAdd(&A.parts_done[s], 1u);
+  arrived = __shfl_sync(0xffffffffu, arrived, 0);
+  if (arrived + 1 != parts) return PartMerge{false, 0ull};
+  __threadfence();
+  static_assert(kMaxParts * kFastTopK <= 128, "a lane merges at most four keys of the parts' lists");
+  unsigned long long k[4];
+#pragma unroll
+  for (int j = 0; j < 4; j++) k[j] = lane + 32u * j < parts * kFastTopK ? __ldcg(pt + lane + 32u * j) : 0ull;
+  best = 0ull;
+  for (uint32_t r = 0; r < K; r++) {
+    unsigned long long m = k[0];
+#pragma unroll
+    for (int j = 1; j < 4; j++) m = k[j] > m ? k[j] : m;
+    const unsigned long long wm = warp_max_u64(m);
+    if (wm != 0ull) {
+      bool gone = false;     // (keys are unique: at most one of the lane's four matches)
+#pragma unroll
+      for (int j = 0; j < 4; j++) if (!gone && k[j] == wm) { k[j] = 0ull; gone = true; }
+    }
+    if (lane == r) best = wm;
+  }
+  return PartMerge{true, best};
+}
+
 // Run by ONE warp while the others score: take the CTA's next spectrum from the queue and leave in shared memory what
 // its iteration would otherwise wait for -- the precursor and candidate ranges, the binned peaks (cp.async) and the
 // occupied-block bitmap with its numbering.
@@ -450,8 +508,7 @@ __device__ __noinline__ void prefetch_spectrum(const ScoreArgs& A, SpecShared& s
   if (lane == 0) vn = atomicAdd(A.work, 1u);
   vn = __shfl_sync(0xffffffffu, vn, 0);
   const uint32_t wn = vn / A.parts;          // work item -> (spectrum, part); sn >= n_spec ends the CTA
-  const uint32_t n_work = A.n_work_dev ? __ldcg(A.n_work_dev) : A.n_work;
-  const uint32_t sn = wn < n_work ? (A.remap ? A.remap[wn] : wn) : A.n_spec;
+  const uint32_t sn = wn < A.n_work ? (A.remap ? A.remap[wn] : wn) : A.n_spec;
   SpecMeta m;
   m.part = vn % A.parts; m.c_lo = 0; m.c_hi = 0;
   m.s = sn; m.pre_blocks = 0; m.nact = 0; m.nt = 0; m.nd = 0; m.npk = 0; m.hbin = -1; m.t0c = 0; m.pk0 = 0;
@@ -484,16 +541,7 @@ __device__ __noinline__ void prefetch_spectrum(const ScoreArgs& A, SpecShared& s
         for (uint32_t k = b0; k <= b1; k++) atomicOr(&bits[k >> 5], 1u << (k & 31));
       }
       __syncwarp();
-      uint32_t run = 0;
-      for (uint32_t base = 0; base < nwords; base += 32) {   // exclusive popcount prefix over the bitmap words
-        const uint32_t i = base + lane;
-        const uint32_t c = i < nwords ? (uint32_t)__popc(bits[i]) : 0u;
-        uint32_t incl = c;
-        for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((int)lane >= o) incl += t; }
-        if (i < nwords) bpre[i] = run + incl - c;
-        run += __shfl_sync(0xffffffffu, incl, 31);
-      }
-      m.nact = run; m.pre_blocks = 1;
+      m.nact = warp_bitmap_prefix(bits, bpre, nwords); m.pre_blocks = 1;
     }
   }
   __syncwarp();
@@ -518,24 +566,9 @@ __device__ __noinline__ void finish_spectrum(const ScoreArgs& A, const ScoreCons
     }
   }
   if (A.parts > 1) {
-    // leave this part's keys; the last part of the spectrum to arrive merges all of them
-    unsigned long long* pt = A.part_top + (size_t)f.s * A.parts * kFastTopK;
-    if (lane < kFastTopK) pt[f.part * kFastTopK + lane] = lane < K ? mine : 0ull;
-    __threadfence();
-    uint32_t arrived = 0;
-    if (lane == 0) arrived = atomicAdd(&A.parts_done[f.s], 1u);
-    arrived = __shfl_sync(0xffffffffu, arrived, 0);
-    if (arrived + 1 != A.parts) return;
-    __threadfence();
-    static_assert(8 * kFastTopK <= 64, "a lane merges at most two keys of the parts' lists");
-    unsigned long long k0 = lane < A.parts * kFastTopK ? __ldcg(pt + lane) : 0ull;
-    unsigned long long k1 = lane + 32 < A.parts * kFastTopK ? __ldcg(pt + lane + 32) : 0ull;
-    mine = 0ull;
-    for (uint32_t r = 0; r < K; r++) {
-      const unsigned long long wm = warp_max_u64(k0 > k1 ? k0 : k1);
-      if (wm != 0ull) { if (k0 == wm) k0 = 0ull; else if (k1 == wm) k1 = 0ull; }
-      if (lane == r) mine = wm;
-    }
+    const PartMerge pm = merge_parts(A, f.s, f.part, A.parts, K, mine);
+    if (!pm.last) return;
+    mine = pm.best;
   }
   if (lane < K) write_psm_row(A, C, f.pr, f.s, lane, mine, f.nt, f.nd, f.t0c);
 }
@@ -544,7 +577,6 @@ __device__ __noinline__ void finish_spectrum(const ScoreArgs& A, const ScoreCons
 // known at compile time); 1: general; 2: general, and spectra are divided into parts (ScoreArgs::parts > 1)
 template <bool HASVAR, int MODE>
 __global__ void __launch_bounds__(kScoreThreads, 1) k_score(const __grid_constant__ ScoreArgs A, const __grid_constant__ ScoreConst C) {
-  if (A.n_work_dev && __ldcg(A.n_work_dev) == 0u) return;            // (launched behind k_score_pipe for the spectra it left: usually none)
   extern __shared__ __align__(16) int32_t tab[];                     // kTileBins
   int64_t* s_score = reinterpret_cast<int64_t*>(tab + kTileBins);    // kCandChunk
   int32_t* s_bin = reinterpret_cast<int32_t*>(s_score + kCandChunk); // 2 x kPeakCap
@@ -559,9 +591,6 @@ __global__ void __launch_bounds__(kScoreThreads, 1) k_score(const __grid_constan
   constexpr uint32_t kPrefetchWarp = NW - 1, kFinishWarp = NW - 2;
   const LaneTab L{C.tq[lane], C.tr[lane], C.vq[lane], C.vr[lane]};   // per-letter (q, r) tables in registers: lane = residue code
   uint32_t my_pairs = 0, my_bytes = 0;   // per thread, summed at the end
-  long long t_last = A.timing ? clock64() : 0;
-  if (tid < 8) sh.tacc[tid] = 0;
-#define MD_TICK(k) do { if (A.timing && tid == 0) { const long long now_ = clock64(); sh.tacc[k] += now_ - t_last; t_last = now_; } } while (0)
 
   if (warp == kPrefetchWarp) prefetch_spectrum(A, sh, 0, s_bin, s_yq);
   if (tid < 2) sh.fin[tid].pending = 0;
@@ -609,22 +638,13 @@ __global__ void __launch_bounds__(kScoreThreads, 1) k_score(const __grid_constan
         for (uint32_t k = b0; k <= b1; k++) atomicOr(&bits[k >> 5], 1u << (k & 31));
       }
       __syncthreads();
-      if (warp == 0) {   // exclusive popcount prefix over the bitmap words
-        uint32_t run = 0;
-        for (uint32_t base = 0; base < nwords; base += 32) {
-          const uint32_t i = base + lane;
-          const uint32_t c = i < nwords ? (uint32_t)__popc(bits[i]) : 0u;
-          uint32_t incl = c;
-          for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((int)lane >= o) incl += t; }
-          if (i < nwords) bpre[i] = run + incl - c;
-          run += __shfl_sync(0xffffffffu, incl, 31);
-        }
+      if (warp == 0) {
+        const uint32_t run = warp_bitmap_prefix(bits, bpre, nwords);
         if (lane == 0) sh.nact = run;
       }
       __syncthreads();
     }
     const uint32_t nact = scored ? (mt.pre_blocks ? mt.nact : sh.nact) : 0;
-    MD_TICK(0);
 
     const bool fast = K <= kFastTopK;   // per-warp running top-k lists, merged by the finish warp while the CTA scores the next spectrum
     // the table of one tile of occupied blocks [cb0, cb0 + cbn) (block-uniform: every thread calls it)
@@ -649,7 +669,6 @@ __global__ void __launch_bounds__(kScoreThreads, 1) k_score(const __grid_constan
         if (tid == 0) { sh.unit = 0; sh.cin = 0; }
       }
       __syncthreads();
-      MD_TICK(2);
       // (2) T as a difference array: every peak adds +y at the first bin of its window (bin-75), -y behind its last
       //     (bin+76), and its own 151*y spike as -151*y at bin / +151*y at bin+1, so that the running sum over the
       //     bins is R[b] = S[b] - 151*y[b] = -T[b].  All four bins lie in occupied blocks (the marking covers
@@ -675,7 +694,6 @@ __global__ void __launch_bounds__(kScoreThreads, 1) k_score(const __grid_constan
         if (cb0 > 0 && cin != 0) atomicAdd(&sh.cin, cin);
       }
       __syncthreads();
-      MD_TICK(3);
       // (3) the scan, in place, negated: every thread owns a contiguous range of 16-byte words (an odd number of them:
       //     the 128-bit accesses of a quarter warp then fall into distinct banks); pass A adds up the ranges, a warp scan
       //     and the per-warp sums give every thread its start value, pass B rescans the range
@@ -698,7 +716,6 @@ __global__ void __launch_bounds__(kScoreThreads, 1) k_score(const __grid_constan
         }
       }
       __syncthreads();
-      MD_TICK(6);
     };
     const bool one_tile = nact <= kTileBlocks;   // the usual case: the table is built once and serves every chunk of candidates
     const uint32_t c_lo = MODE == 2 ? mt.c_lo : 0u, c_hi = MODE == 2 ? mt.c_hi : ncand;     // this work item's candidates (the whole spectrum unless it was split)
@@ -724,12 +741,7 @@ __global__ void __launch_bounds__(kScoreThreads, 1) k_score(const __grid_constan
           }
         }
         __syncthreads();
-        if (warp == 0) {  // exclusive prefix over the 64 buckets
-          const uint32_t h0 = sh.hist[2 * lane], h1 = sh.hist[2 * lane + 1];
-          uint32_t incl = h0 + h1;
-          for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((int)lane >= o) incl += t; }
-          sh.hist[2 * lane] = incl - h0 - h1; sh.hist[2 * lane + 1] = incl - h1;
-        }
+        if (warp == 0) warp_hist64_prefix(sh.hist);
         __syncthreads();
         if (scored) {
 #pragma unroll
@@ -740,7 +752,6 @@ __global__ void __launch_bounds__(kScoreThreads, 1) k_score(const __grid_constan
         }
       }
       // (visible to the scoring warps after the table-build barriers)
-      MD_TICK(1);
       if (scored && cn) {
         for (uint32_t cb0 = 0; cb0 < nact; cb0 += kTileBlocks) {       // tiles of occupied blocks (usually one)
           const uint32_t cbn = min(kTileBlocks, nact - cb0);
@@ -765,7 +776,6 @@ __global__ void __launch_bounds__(kScoreThreads, 1) k_score(const __grid_constan
             }
           }
           __syncthreads();
-          MD_TICK(4);
         }
       }
       // ---- raw scores of every candidate (on request)
@@ -833,15 +843,12 @@ __global__ void __launch_bounds__(kScoreThreads, 1) k_score(const __grid_constan
         FinRecord f; f.pr = pr; f.t0c = t0c; f.s = s; f.nt = nt; f.nd = nd; f.pending = 1; f.ranked = (scored && K) ? 1u : 0u; f.part = mt.part;
         sh.fin[slot] = f;
       }
-      MD_TICK(5);
     } else {
       for (uint32_t r = tid; r < K; r += kScoreThreads) write_psm_row(A, C, pr, s, r, scored ? sh.top[r] : 0ull, nt, nd, t0c);
       if (tid == 0) sh.fin[slot].pending = 0;
       __syncthreads();
-      MD_TICK(5);
     }
   }
-  if (A.timing && tid == 0) for (int k = 0; k < 8; k++) atomicAdd(&A.timing[k], (unsigned long long)sh.tacc[k]);
   unsigned long long wp = my_pairs, wb = my_bytes;
   for (int o = 16; o; o >>= 1) { wp += __shfl_xor_sync(0xffffffffu, wp, o); wb += __shfl_xor_sync(0xffffffffu, wb, o); }
   if (lane == 0 && wp) { atomicAdd(&A.stat64[0], wp); atomicAdd(&A.stat64[1], wb); }
@@ -864,13 +871,15 @@ __global__ void __launch_bounds__(kScoreThreads, 1) k_score(const __grid_constan
 //   k_score_pipe    one persistent CTA per SM.  A LOADER warp takes the next spectrum from the queue, finds room for its
 //                   table in a RING of shared-memory blocks (two spectra are resident whenever their tables fit side by
 //                   side) and issues cp.async.bulk copies of map, table and candidate order that complete on the slot's
-//                   mbarrier.  23 SCORER warps each pull 32-candidate units of the current spectrum, keep their K best
-//                   keys in registers, and when the units run out leave them in shared memory and walk on to the next
-//                   spectrum if its table has landed; the last warp to leave a spectrum merges the lists, writes the PSM
-//                   rows and releases the slot (empty mbarrier).
-// Same arithmetic as k_score (score_one): bit-identical rows.  Batches this path does not take (top_k > 8, spectra split
-// into parts) use k_score; a spectrum it cannot hold (more than 512 binned peaks, a block map beyond 4096 entries, a table
-// beyond the ring) goes onto a list that k_score works off afterwards.
+//                   mbarrier.  The other warps (19 at 640 threads) SCORE: each pulls 32-candidate units of the current
+//                   spectrum, keeps its K best keys in registers, and when the units run out leaves them in shared memory
+//                   and walks on to the next spectrum if its table has landed; the last warp to leave a spectrum merges
+//                   the lists, releases the slot (empty mbarrier) and then writes the PSM rows -- for a spectrum split
+//                   into parts, only the last part to finish does, after merging the parts' lists (merge_parts).
+// Same arithmetic as k_score (score_one): bit-identical rows.  Batches this path does not take (top_k > 8, a fixed
+// N-terminus modification, MD_SCORE_CLASSIC, split batches under MD_SCORE_SPLIT_CLASSIC) use k_score; a spectrum it cannot
+// hold (more than 1024 binned peaks, a block map beyond 4096 entries, a table record beyond the ring) goes onto the list
+// that k_build_tables leaves, and k_score works that list off on the side stream beside this kernel.
 #ifndef MD_PIPE_THREADS
 #define MD_PIPE_THREADS 640     // swept on C2 / C3: 448 .. 1024 threads; 640 (19 scorer warps at up to 102 registers) is the fastest
 #endif
@@ -883,7 +892,6 @@ constexpr uint32_t kPoolBlocks = 856;      // most 64-bin blocks (the all-zero b
 constexpr uint32_t kRingBytes = 214 * 1024; // shared-memory ring that holds the table records (block map + table) of two spectra
 constexpr uint32_t kPipeEnd = 0xFFFFFFFFu, kTabLeft = 0xFFFFFFFFu;
 constexpr uint32_t kTabThreads = 256;
-constexpr uint32_t kPipeMaxParts = 16;     // most work items the pipelined kernel splits a spectrum into
 
 // where a spectrum's table record lies in the pool.  nblk == 0: the spectrum is not scored (too few peaks); nact == kTabLeft: k_score takes it
 struct TabDesc { unsigned long long off; uint32_t nact, nblk; };
@@ -893,7 +901,7 @@ constexpr size_t kTabMaxBytes = (((size_t)kPMapCap + 1) * 2 + 15) / 16 * 16 + (s
 __global__ void __launch_bounds__(kTabThreads) k_build_tables(const uint64_t* __restrict__ peak_off, const int32_t* __restrict__ pk_bin, const int32_t* __restrict__ pk_yq,
                                                               const uint32_t* __restrict__ pk_count, const int32_t* __restrict__ pk_hbin, uint8_t* __restrict__ pool,
                                                               unsigned long long* __restrict__ pool_top, TabDesc* __restrict__ desc,
-                                                              uint32_t* __restrict__ left_list, uint32_t* __restrict__ left_n) {
+                                                              uint32_t* __restrict__ left_list, uint32_t* __restrict__ n_left) {
   __shared__ int32_t s_bin[kPPeaks], s_yq[kPPeaks];
   __shared__ uint32_t s_bits[kPMapCap / 32], s_pre[kPMapCap / 32];
   __shared__ uint16_t s_blk[kPoolBlocks];
@@ -906,7 +914,7 @@ __global__ void __launch_bounds__(kTabThreads) k_build_tables(const uint64_t* __
   const uint32_t NB = hbin >= 0 ? (uint32_t)hbin + kXcorrOffset + 1 : 0u;       // table bins [0, NB)
   const uint32_t nblk = (NB + kBlk - 1) >> kBlkShift, nwords = (nblk + 31) >> 5;
   if (hbin < 0 || NB > kMaxBins) { if (tid == 0) desc[s] = TabDesc{0ull, 0u, 0u}; return; }
-  if (npk > kPPeaks || nblk > kPMapCap) { if (tid == 0) { desc[s] = TabDesc{0ull, kTabLeft, nblk}; left_list[atomicAdd(left_n, 1u)] = s; } return; }
+  if (npk > kPPeaks || nblk > kPMapCap) { if (tid == 0) { desc[s] = TabDesc{0ull, kTabLeft, nblk}; left_list[atomicAdd(n_left, 1u)] = s; } return; }
   for (uint32_t i = tid; i < npk; i += kTabThreads) { s_bin[i] = pk_bin[pk0 + i]; s_yq[i] = pk_yq[pk0 + i]; }
   for (uint32_t i = tid; i < nwords; i += kTabThreads) s_bits[i] = 0;
   __syncthreads();
@@ -916,16 +924,8 @@ __global__ void __launch_bounds__(kTabThreads) k_build_tables(const uint64_t* __
     for (uint32_t k = b0; k <= b1; k++) atomicOr(&s_bits[k >> 5], 1u << (k & 31));
   }
   __syncthreads();
-  if (tid < 32) {   // exclusive popcount prefix over the bitmap words
-    uint32_t run = 0;
-    for (uint32_t w0 = 0; w0 < nwords; w0 += 32) {
-      const uint32_t i = w0 + lane;
-      const uint32_t c = i < nwords ? (uint32_t)__popc(s_bits[i]) : 0u;
-      uint32_t incl = c;
-      for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((int)lane >= o) incl += t; }
-      if (i < nwords) s_pre[i] = run + incl - c;
-      run += __shfl_sync(0xffffffffu, incl, 31);
-    }
+  if (tid < 32) {
+    const uint32_t run = warp_bitmap_prefix(s_bits, s_pre, nwords);
     if (lane == 0) {
       s_nact = run;
       if (run + 1u <= kPoolBlocks && tab_map_bytes(nblk) + (run + 1u) * kBlk * 4u <= kRingBytes) s_base = atomicAdd(pool_top, (unsigned long long)tab_map_bytes(nblk) + (unsigned long long)(run + 1u) * kBlk * 4u);
@@ -933,7 +933,7 @@ __global__ void __launch_bounds__(kTabThreads) k_build_tables(const uint64_t* __
   }
   __syncthreads();
   const uint32_t nact = s_nact;
-  if (nact + 1u > kPoolBlocks || tab_map_bytes(nblk) + (nact + 1u) * kBlk * 4u > kRingBytes) { if (tid == 0) { desc[s] = TabDesc{0ull, kTabLeft, nblk}; left_list[atomicAdd(left_n, 1u)] = s; } return; }
+  if (nact + 1u > kPoolBlocks || tab_map_bytes(nblk) + (nact + 1u) * kBlk * 4u > kRingBytes) { if (tid == 0) { desc[s] = TabDesc{0ull, kTabLeft, nblk}; left_list[atomicAdd(n_left, 1u)] = s; } return; }
   const unsigned long long base = s_base;
   if (tid == 0) desc[s] = TabDesc{base, nact, nblk};
   // ---- block map: entry = (block of the record << 6) | 63, block 0 of the record = the all-zero block every miss reads
@@ -1004,7 +1004,7 @@ __global__ void k_pair_schedule(const uint32_t* __restrict__ asc, uint32_t n, bo
 // candidates of every spectrum with at most kPOrder of them, counting-sorted by length (longest first) -> order[s * kPOrder + i]
 __global__ void __launch_bounds__(256) k_cand_order(const ScoreArgs A, uint32_t n_per, uint16_t* __restrict__ order) {
   __shared__ uint32_t hist[64];
-  const uint32_t s = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+  const uint32_t s = blockIdx.x, tid = threadIdx.x;
   const uint64_t t0c = A.cand_off[s];
   const uint32_t nt = (uint32_t)(A.cand_off[s + 1] - t0c), nd = A.dec_count ? A.dec_count[s] : 0u, ncand = nt + nd;
   if (ncand > kPOrder || A.pk_hbin[s] < 0) return;
@@ -1019,12 +1019,7 @@ __global__ void __launch_bounds__(256) k_cand_order(const ScoreArgs A, uint32_t 
 #pragma unroll
   for (uint32_t h = 0; h < kPOrder / 256; h++) if (tid + h * 256 < ncand) atomicAdd(&hist[63u - min((uint32_t)lens[h], 63u)], 1u);
   __syncthreads();
-  if (tid < 32) {  // exclusive prefix over the 64 buckets
-    const uint32_t h0 = hist[2 * lane], h1 = hist[2 * lane + 1];
-    uint32_t incl = h0 + h1;
-    for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((int)lane >= o) incl += t; }
-    hist[2 * lane] = incl - h0 - h1; hist[2 * lane + 1] = incl - h1;
-  }
+  if (tid < 32) warp_hist64_prefix(hist);
   __syncthreads();
   uint16_t* out = order + (size_t)s * kPOrder;
 #pragma unroll
@@ -1032,39 +1027,6 @@ __global__ void __launch_bounds__(256) k_cand_order(const ScoreArgs A, uint32_t 
     const uint32_t v = tid + h * 256;
     if (v < ncand) out[atomicAdd(&hist[63u - min((uint32_t)lens[h], 63u)], 1u)] = (uint16_t)v;
   }
-}
-
-// A spectrum split into parts: the work item leaves its K best keys; the last part of the spectrum to arrive merges them all
-// (lane r returns with the spectrum's r-th best key) and writes the rows.  False: another part will.
-__device__ __noinline__ bool merge_parts(const ScoreArgs& A, uint32_t s, uint32_t part, uint32_t parts, uint32_t K, unsigned long long& best) {
-  const uint32_t lane = threadIdx.x & 31;
-  unsigned long long* pt = A.part_top + (size_t)s * parts * kFastTopK;
-  if (lane < kFastTopK) pt[part * kFastTopK + lane] = lane < K ? best : 0ull;
-  __threadfence();
-  __syncwarp();
-  uint32_t arrived = 0;
-  if (lane == 0) arrived = atomicAdd(&A.parts_done[s], 1u);
-  arrived = __shfl_sync(0xffffffffu, arrived, 0);
-  if (arrived + 1 != parts) return false;
-  __threadfence();
-  static_assert(kPipeMaxParts * kFastTopK <= 128, "a lane merges at most four keys of the parts' lists");
-  unsigned long long k[4];
-#pragma unroll
-  for (int j = 0; j < 4; j++) k[j] = lane + 32u * j < parts * kFastTopK ? __ldcg(pt + lane + 32u * j) : 0ull;
-  best = 0ull;
-  for (uint32_t r = 0; r < K; r++) {
-    unsigned long long m = k[0];
-#pragma unroll
-    for (int j = 1; j < 4; j++) m = k[j] > m ? k[j] : m;
-    const unsigned long long wm = warp_max_u64(m);
-    if (wm != 0ull) {
-      bool gone = false;     // (keys are unique: at most one of the lane's four matches)
-#pragma unroll
-      for (int j = 0; j < 4; j++) if (!gone && k[j] == wm) { k[j] = 0ull; gone = true; }
-    }
-    if (lane == r) best = wm;
-  }
-  return true;
 }
 
 struct PipeSlot {
@@ -1079,8 +1041,6 @@ struct PipeShared {
   PipeSlot slot[2];
   unsigned long long ready[2], empty[2];                       // mbarriers
   unsigned long long wtop[2][kScoreWarps][kFastTopK];
-  uint32_t state[2];   // (diagnosis) 0 = the slot's spectrum has left, 1 = the loader is on its next one, 2 = copies issued
-  uint32_t blocked[2]; // (diagnosis) the loader is waiting for the ring to drain before it can place this slot's record
 };
 
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
@@ -1142,8 +1102,6 @@ __global__ void __launch_bounds__(kPipeThreads, 1) k_score_pipe(const __grid_con
     // =============================================================================== loader (one lane works; the warp keeps it company)
     if (lane == 0) {
       uint32_t prev_need = 0;                          // ring bytes of the previous spectrum's record (it lies at the other end of the ring)
-      long long t_wait = 0;
-      const long long t_begin = A.timing ? clock64() : 0;
       uint32_t pend = kPipeEnd;                        // second spectrum of the pair that was drawn last
       for (uint32_t q = 0;; q++) {
         const uint32_t b = q & 1, use = q >> 1;
@@ -1165,13 +1123,8 @@ __global__ void __launch_bounds__(kPipeThreads, 1) k_score_pipe(const __grid_con
         TabDesc d{0ull, 0u, 0u};
         if (!end) { pr = A.prec[s]; t0c = A.cand_off[s]; nt = (uint32_t)(A.cand_off[s + 1] - t0c); nd = A.dec_count ? A.dec_count[s] : 0u; d = T.desc[s]; }
         const uint32_t ncand = nt + nd;
-        if (use > 0) { const long long t0 = A.timing ? clock64() : 0; mbar_wait(&sh.empty[b], (use - 1) & 1); if (A.timing) t_wait += clock64() - t0; }   // the slot's previous spectrum has left
-        if (A.timing) sh.state[b] = 1;
-        if (end) {
-          S.s = kPipeEnd; __threadfence_block(); mbar_arrive(&sh.ready[b]);
-          if (A.timing) { const long long all = clock64() - t_begin; atomicAdd(&A.timing[0], (unsigned long long)(all - t_wait)); atomicAdd(&A.timing[1], (unsigned long long)t_wait); }
-          break;
-        }
+        if (use > 0) mbar_wait(&sh.empty[b], (use - 1) & 1);   // the slot's previous spectrum has left
+        if (end) { S.s = kPipeEnd; __threadfence_block(); mbar_arrive(&sh.ready[b]); break; }
         bool scored = d.nblk != 0u, left = false;
         if (scored && ncand > 0xFFFFFFu) { *A.error = 1; scored = false; }
         if (scored && d.nact == kTabLeft) { left = true; scored = false; }
@@ -1181,13 +1134,7 @@ __global__ void __launch_bounds__(kPipeThreads, 1) k_score_pipe(const __grid_con
           // ---- room for the record in the ring: records alternate between its two ends, so two spectra are resident whenever
           //      their records fit side by side; if they do not, the previous spectrum has to leave first
           need = tab_map_bytes(d.nblk) + (d.nact + 1u) * kBlk * 4u;
-          if (prev_need + need > kRingBytes && q > 0) {
-            const long long t0 = A.timing ? clock64() : 0;
-            if (A.timing) sh.blocked[b] = 1;
-            mbar_wait(&sh.empty[b ^ 1u], ((q - 1) >> 1) & 1);
-            if (A.timing) sh.blocked[b] = 0;
-            if (A.timing) { t_wait += clock64() - t0; atomicAdd(&A.timing[6], 1ull); }
-          }
+          if (prev_need + need > kRingBytes && q > 0) mbar_wait(&sh.empty[b ^ 1u], ((q - 1) >> 1) & 1);
           base = b ? kRingBytes - need : 0u;
         }
         S.pr = pr; S.t0c = t0c; S.s = s; S.nt = nt; S.nd = nd; S.ncand = ncand; S.nunits = (ncand + 31) >> 5; S.nblk = d.nblk;
@@ -1210,8 +1157,6 @@ __global__ void __launch_bounds__(kPipeThreads, 1) k_score_pipe(const __grid_con
           }
           if (sorted) bulk_g2s(s_order0 + b * kPOrder, T.order + (size_t)s * kPOrder, obytes, &sh.ready[b]);
           prev_need = need;
-          if (A.timing) sh.state[b] = 2;
-          if (A.timing) { const long long t0 = clock64(); mbar_wait(&sh.ready[b], use & 1); atomicAdd(&A.timing[7], (unsigned long long)(clock64() - t0)); atomicAdd(&A.timing[4], (unsigned long long)need); }   // (diagnosis: how long the copies take)
         } else {
           mbar_arrive(&sh.ready[b]);
           prev_need = 0;
@@ -1225,16 +1170,9 @@ __global__ void __launch_bounds__(kPipeThreads, 1) k_score_pipe(const __grid_con
   const LaneTab L{C.tq[lane], C.tr[lane], C.vq[lane], C.vr[lane]};   // per-letter (q, r) tables in registers: lane = residue code
   uint32_t my_pairs = 0, my_bytes = 0;
   const uint32_t K = C.top_k;
-  long long s_wait = 0, w_cause[4] = {0, 0, 0, 0};
-  const long long s_begin = A.timing ? clock64() : 0;
   for (uint32_t q = 0;; q++) {
     const uint32_t b = q & 1, use = q >> 1;
-    {
-      const long long t0 = A.timing ? clock64() : 0;
-      const uint32_t st0 = A.timing ? ((volatile uint32_t*)sh.state)[b] : 0u, bl0 = A.timing ? ((volatile uint32_t*)sh.blocked)[b] : 0u;
-      mbar_wait_warp(&sh.ready[b], use & 1);
-      if (A.timing) { const long long dt = clock64() - t0; s_wait += dt; if (bl0) w_cause[3] += dt; else w_cause[st0 < 3 ? st0 : 2] += dt; }
-    }
+    mbar_wait_warp(&sh.ready[b], use & 1);
     PipeSlot& S = sh.slot[b];
     const uint32_t s = S.s;
     if (s == kPipeEnd) break;
@@ -1324,20 +1262,16 @@ __global__ void __launch_bounds__(kPipeThreads, 1) k_score_pipe(const __grid_con
       }
       // the slot is free as soon as the lists are merged: the rows (an FP64 division each, thousands of cycles on this part)
       // are written from registers while the loader already brings the slot's next spectrum
-#ifdef MD_PIPE_LATE_RELEASE
-      if (lane < K && !left_out) write_psm_row(A, C, pr, s, lane, best, nt, nd, t0c);
       __syncwarp();
-      if (lane == 0) { S.done = 0; if (A.timing) sh.state[b] = 0; __threadfence_block(); mbar_arrive(&sh.empty[b]); }
-#else
-      __syncwarp();
-      if (lane == 0) { S.done = 0; if (A.timing) sh.state[b] = 0; __threadfence_block(); mbar_arrive(&sh.empty[b]); }
-      if (T.parts > 1 && !left_out) { if (!merge_parts(A, s, S_part, T.parts, K, best)) continue; }
+      if (lane == 0) { S.done = 0; __threadfence_block(); mbar_arrive(&sh.empty[b]); }
+      if (T.parts > 1 && !left_out) {
+        const PartMerge pm = merge_parts(A, s, S_part, T.parts, K, best);
+        if (!pm.last) continue;
+        best = pm.best;
+      }
       if (lane < K && !left_out) write_psm_row(A, C, pr, s, lane, best, nt, nd, t0c);
-#endif
     }
   }
-  if (A.timing && tid == 0) { for (int k = 0; k < 4; k++) atomicAdd(&A.timing[8 + k], (unsigned long long)w_cause[k]); }
-  if (A.timing && tid == 0) { const long long all = clock64() - s_begin; atomicAdd(&A.timing[2], (unsigned long long)s_wait); atomicAdd(&A.timing[3], (unsigned long long)(all - s_wait)); }
   unsigned long long wp = my_pairs, wb = my_bytes;
   for (int o = 16; o; o >>= 1) { wp += __shfl_xor_sync(0xffffffffu, wp, o); wb += __shfl_xor_sync(0xffffffffu, wb, o); }
   if (lane == 0 && wp) { atomicAdd(&A.stat64[0], wp); atomicAdd(&A.stat64[1], wb); }
@@ -1373,6 +1307,23 @@ bool classic_only(const md_ctx* ctx) {
   return false;
 }
 
+constexpr size_t kScoreSmem = (size_t)kTileBins * sizeof(int32_t) + (size_t)kCandChunk * sizeof(int64_t) + 2 * (size_t)kPeakCap * 8 + (size_t)kCandChunk * 2 +
+                              ((size_t)kMapCap + 2) * 2;
+
+// k_score over the work items of A on `stream`, instantiated for the batch: HASVAR = any variable modification, MODE from
+// A.parts and `single` (every spectrum of the batch fits one chunk of candidates)
+void launch_k_score(md_ctx* ctx, cudaStream_t stream, uint32_t grid, const ScoreArgs& A, const ScoreConst& C, bool has_var, bool single) {
+  auto go = [&](auto kernel) {
+    MD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScoreSmem));
+    kernel<<<grid, kScoreThreads, kScoreSmem, stream>>>(A, C);
+    ctx->launches++;
+    MD_CUDA(cudaGetLastError());
+  };
+  const int mode = A.parts > 1 ? 2 : (single ? 0 : 1);
+  if (has_var) { if (mode == 2) go(k_score<true, 2>); else if (mode == 0) go(k_score<true, 0>); else go(k_score<true, 1>); }
+  else { if (mode == 2) go(k_score<false, 2>); else if (mode == 0) go(k_score<false, 0>); else go(k_score<false, 1>); }
+}
+
 }  // namespace
 
 void precursors_dev(md_ctx* ctx, const SpectraDev& S, const md_search_params& p, uint32_t id_base) {
@@ -1391,8 +1342,9 @@ void score_prepare_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const
   const int64_t w = (int64_t)llround(p.fragment_tolerance * 1000000.0);
   W.pk_bin.need(n_peaks + 1); W.pk_yq.need(n_peaks + 1); W.pk_count.need(n + 1); W.pk_hbin.need(n + 1);
   DevBuf<int>& d_flag = W.t_unsorted; d_flag.need(4);
-  W.stat64.need(32);
+  W.stat64.need(5);
   const bool tables = p.top_k <= kFastTopK && !classic_only(ctx);
+  W.tables_built = tables;
   if (tables) { W.tab_pool.need((size_t)n * kTabMaxBytes + 256); W.tab_desc.need((size_t)n * sizeof(TabDesc) + 16); W.left_list.need(n + 2); }
   cudaStream_t main = ctx->stream, side = ctx->stream2;
   MD_CUDA(cudaEventRecord(ctx->ev_fork, main));
@@ -1418,11 +1370,10 @@ void score_prepare_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const
   ctx->stream = main;
 }
 
-void score_run_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const md_search_params& p, uint32_t n_per, md_psm* psm_dev, bool want_all) {
+void score_run_dev(md_ctx* ctx, const SpectraDev& S, const md_search_params& p, uint32_t n_per, md_psm* psm_dev, bool want_all) {
   IdentifyWorkspace& W = ctx->ws;
   const uint32_t n = S.n;
   if (!n) return;
-  (void)n_peaks;
   const int64_t w = (int64_t)llround(p.fragment_tolerance * 1000000.0);
   const uint32_t mfc = p.max_fragment_charge ? p.max_fragment_charge : 3;
   MD_REQUIRE(mfc <= 3, MD_ERR_UNSUPPORTED, "max_fragment_charge > 3 (the reference fixes it to 3: comet_parameter.rs:55)");
@@ -1433,8 +1384,7 @@ void score_run_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const md_
   int h_pre[4] = {0, 0, 0, 0};
   uint32_t n_left = 0;           // spectra k_build_tables found too dense for the pipelined kernel
   MD_CUDA(cudaMemcpyAsync(h_pre, d_flag.p, sizeof(h_pre), cudaMemcpyDeviceToHost, ctx->stream));
-  const bool tables_built = p.top_k <= kFastTopK && !classic_only(ctx);
-  if (tables_built) MD_CUDA(cudaMemcpyAsync(&n_left, W.left_list.p + n, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (W.tables_built) MD_CUDA(cudaMemcpyAsync(&n_left, W.left_list.p + n, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
   // ---- K4
   ScoreConst C;
   memset(&C, 0, sizeof(C));
@@ -1468,28 +1418,30 @@ void score_run_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const md_
   // Few spectra with very many candidates each (open searches) would leave SMs idle and make one CTA walk hundreds of
   // chunks: split every spectrum into `parts` work items (contiguous ranges of candidate chunks; each builds the table
   // itself, which is cheap beside the chunks), about two items per SM.  MD_SCORE_SPLIT_MIN = candidates per spectrum
-  // (batch average) from which that is done (tests lower it).
-  const bool pipe_path = p.top_k <= kFastTopK && !classic_only(ctx) && getenv("MD_SCORE_SPLIT_CLASSIC") == nullptr;
+  // (batch average) from which that is done (tests lower it).  Only the per-warp top-k lists (top_k <= 8) merge across parts.
+  const bool split_classic = getenv("MD_SCORE_SPLIT_CLASSIC") != nullptr;   // (tests: a split batch goes through k_score)
   uint32_t parts = 1;
-  {
-    uint64_t n_cand = (uint64_t)n * n_per, split_min = 16ull * kCandChunk;
-    n_cand += n_targets;
+  if (p.top_k <= kFastTopK) {
+    const uint64_t n_cand = (uint64_t)n * n_per + n_targets;
+    uint64_t split_min = 16ull * kCandChunk;
     if (const char* env = getenv("MD_SCORE_SPLIT_MIN")) split_min = std::max<long long>(1, atoll(env));
-    if (n < (uint32_t)ctx->n_sm && p.top_k <= kFastTopK && n_cand / n >= split_min)
+    if (n < (uint32_t)ctx->n_sm && n_cand / n >= split_min)
       parts = std::min<uint32_t>(std::min<uint32_t>(8u, (2u * (uint32_t)ctx->n_sm + n - 1) / n), (uint32_t)((n_cand / n + kCandChunk - 1) / kCandChunk));
     parts = std::max(parts, 1u);
-    // the pipelined kernel merges up to kPipeMaxParts lists: of the part counts that leave every scorer warp a few units, the one
-    // whose items fill whole rounds of the persistent CTAs best
-    if (parts > 1 && pipe_path) {
+    // the pipelined kernel: of the part counts that leave every scorer warp a few units, the one whose items fill whole rounds
+    // of the persistent CTAs best
+    if (parts > 1 && W.tables_built && !split_classic) {
       const uint64_t units = (n_cand / n + 31) / 32;
       double best_fill = 0;
-      for (uint32_t k = parts; k <= kPipeMaxParts && units / k >= 8ull * kScoreWarps; k++) {
+      for (uint32_t k = parts; k <= kMaxParts && units / k >= 8ull * kScoreWarps; k++) {
         const double rounds = (double)n * k / ctx->n_sm, fill = rounds / std::ceil(rounds);
         if (fill > best_fill + 0.02) { best_fill = fill; parts = k; }
       }
     }
-    if (const char* env = getenv("MD_SCORE_PARTS")) parts = std::min<uint32_t>(std::max(1, atoi(env)), pipe_path ? kPipeMaxParts : 8u);   // (tests)
+    if (const char* env = getenv("MD_SCORE_PARTS")) parts = std::min<uint32_t>(std::max(1, atoi(env)), kMaxParts);   // (tests)
   }
+  // the pipelined kernel (builders + scorers) takes every batch whose table records were built, unless a split batch is sent to k_score
+  const bool pipe = W.tables_built && (parts == 1 || !split_classic);
   const uint32_t grid = std::min<uint32_t>(n * parts, (uint32_t)ctx->n_sm);
   const uint32_t max_nblk = h_pre[2] >= 0 ? ((uint32_t)h_pre[2] + kXcorrOffset + 1 + kBlk - 1) / kBlk : 0;
   uint32_t gstride = 0;
@@ -1500,37 +1452,23 @@ void score_run_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const md_
   DevBuf<uint32_t>& work = W.counters; work.need(4);
   MD_CUDA(cudaMemsetAsync(work.p, 0, 4 * sizeof(uint32_t), ctx->stream));
   MD_CUDA(cudaMemsetAsync(W.stat64.p, 0, 4 * sizeof(unsigned long long), ctx->stream));                    // [0..1] statistics; [4] = the table pool's fill (score_prepare_dev)
-  MD_CUDA(cudaMemsetAsync(W.stat64.p + 8, 0, 24 * sizeof(unsigned long long), ctx->stream));
-  const bool timing = getenv("MD_SCORE_TIMING") != nullptr;
   ScoreArgs A;
   A.prec = W.prec.p; A.n_spec = n; A.peak_off = S.peak_off; A.pk_bin = W.pk_bin.p; A.pk_yq = W.pk_yq.p; A.pk_count = W.pk_count.p; A.pk_hbin = W.pk_hbin.p;
   A.cand_off = W.cand_off.p; A.cand_desc = W.cand_desc.p; A.cand_mask = W.cand_mask.p; A.cand_w = W.cand_w.p; A.cand_pep = W.cand_pep.p;
   A.idx_rows = ctx->index.rows.p;
   A.dec_slots = (uint64_t)n * n_per; A.dec_rows = W.dec_rows.p; A.dec_len = W.dec_len.p; A.dec_mask = W.dec_mask.p; A.dec_w = W.dec_w.p; A.dec_count = n_per ? W.dec_count.p : nullptr;
   A.tscore = want_all ? W.tscore.p : nullptr; A.dscore = want_all ? W.dscore.p : nullptr; A.psm = psm_dev; A.work = work.p; A.stat64 = W.stat64.p;
-  A.error = d_flag.p + 1; A.timing = timing ? W.stat64.p + 8 : nullptr;
+  A.error = d_flag.p + 1;
   A.gmap = gstride ? W.gmap.p : nullptr; A.gbits = gstride ? W.gbits.p : nullptr; A.gmap_stride = gstride;
   A.parts = parts; A.part_top = nullptr; A.parts_done = nullptr;
-  A.n_work = n; A.remap = nullptr; A.left_list = nullptr; A.left_n = nullptr; A.n_work_dev = nullptr;
+  A.n_work = n; A.remap = nullptr;
   if (parts > 1) {
     W.part_top.need((size_t)n * parts * kFastTopK); W.parts_done.need(n);
     MD_CUDA(cudaMemsetAsync(W.parts_done.p, 0, n * sizeof(uint32_t), ctx->stream));
     A.part_top = W.part_top.p; A.parts_done = W.parts_done.p;
   }
-  const size_t smem = (size_t)kTileBins * sizeof(int32_t) + (size_t)kCandChunk * sizeof(int64_t) + 2 * (size_t)kPeakCap * 8 + (size_t)kCandChunk * 2 +
-                      ((size_t)kMapCap + 2) * 2;
-  MD_CUDA(cudaEventRecord(ctx->ev[6], ctx->stream));
-  auto launch = [&](auto kernel) {
-    MD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    MD_LAUNCH(ctx, kernel, grid, kScoreThreads, smem, A, C);
-  };
   const bool single = parts == 1 && h_pre[3] <= (int)kCandChunk;     // every spectrum fits one chunk of candidates
-  auto launch_classic = [&]() {
-    if (has_var) { if (parts > 1) launch(k_score<true, 2>); else if (single) launch(k_score<true, 0>); else launch(k_score<true, 1>); }
-    else { if (parts > 1) launch(k_score<false, 2>); else if (single) launch(k_score<false, 0>); else launch(k_score<false, 1>); }
-  };
-  // the pipelined kernel (builders + scorers) takes whole-spectrum work items with at most 8 PSM rows; MD_SCORE_CLASSIC=1 forces k_score
-  const bool pipe = p.top_k <= kFastTopK && !classic_only(ctx) && (parts == 1 || pipe_path);
+  MD_CUDA(cudaEventRecord(ctx->ev[6], ctx->stream));
   if (pipe) {
     // the table records are there (score_prepare_dev); the length-sorted candidate order and the schedule, each by the whole GPU at once
     W.cand_order.need((size_t)n * kPOrder + 16);
@@ -1541,32 +1479,21 @@ void score_run_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const md_
     cubx_sort_pairs<uint32_t, uint32_t>(ctx, W.sched_key.p, W.sched_key.p + n, W.sched_val.p, W.sched_val.p + n, n);
     MD_LAUNCH(ctx, k_pair_schedule, blocks((n + 1) / 2), 256, 0, W.sched_val.p + n, n, parts > 1, W.sched.p);
     MD_CUDA(cudaEventRecord(ctx->ev[6], ctx->stream));
+    // spectra too dense for the pipelined kernel (more binned peaks / a larger block map / a larger table record than it stages):
+    // k_score works them off on the side stream, beside the pipelined kernel, whose persistent CTAs leave it g2 SMs (its CTAs
+    // would otherwise wait for the first of them to end)
+    const uint32_t g2 = n_left ? std::min<uint32_t>(std::min<uint32_t>(n_left, grid), std::max<uint32_t>(1u, grid / 8)) : 0u;
     if (n_left) {
-      // spectra too dense for the pipelined kernel (more binned peaks / a larger block map / a larger table record than it stages):
-      // k_score works them off on the side stream, beside the pipelined kernel (one CTA's worth of an SM for a moment)
       MD_CUDA(cudaStreamWaitEvent(ctx->stream2, ctx->ev[6], 0));
       ScoreArgs A2 = A;
       A2.n_work = n_left; A2.remap = W.left_list.p; A2.work = work.p + 2; A2.parts = 1;
-      const uint32_t g2 = std::min<uint32_t>(std::min<uint32_t>(n_left, grid), std::max<uint32_t>(1u, grid / 8));
-      cudaStream_t main = ctx->stream;
-      ctx->stream = ctx->stream2;
-      try {
-        auto launch2 = [&](auto kernel) {
-          MD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-          MD_LAUNCH(ctx, kernel, g2, kScoreThreads, smem, A2, C);
-        };
-        if (has_var) { if (single) launch2(k_score<true, 0>); else launch2(k_score<true, 1>); }
-        else { if (single) launch2(k_score<false, 0>); else launch2(k_score<false, 1>); }
-        MD_CUDA(cudaEventRecord(ctx->ev_prep, ctx->stream2));
-      } catch (...) { ctx->stream = main; throw; }
-      ctx->stream = main;
+      launch_k_score(ctx, ctx->stream2, g2, A2, C, has_var, single);
+      MD_CUDA(cudaEventRecord(ctx->ev_prep, ctx->stream2));
       if (ctx->trace) fprintf(stderr, "[md_trace]   score: %u of %u spectra left to k_score\n", n_left, n);
     }
     const PipeArgs PA{reinterpret_cast<const TabDesc*>(W.tab_desc.p), W.tab_pool.p, W.cand_order.p, W.sched.p, parts};
     auto launch_pipe = [&](auto kernel) {
       MD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPipeSmem));
-      // (the persistent CTAs leave an SM to each CTA of the k_score launch beside them: it would otherwise wait for the first of them to end)
-      const uint32_t g2 = n_left ? std::min<uint32_t>(std::min<uint32_t>(n_left, grid), std::max<uint32_t>(1u, grid / 8)) : 0u;
       MD_LAUNCH(ctx, kernel, grid > g2 ? grid - g2 : grid, kPipeThreads, kPipeSmem, A, C, PA);
     };
     if (has_var) launch_pipe(k_score_pipe<true>); else launch_pipe(k_score_pipe<false>);
@@ -1584,7 +1511,7 @@ void score_run_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const md_
                                na[na.size() / 10], na[na.size() / 2], na[na.size() * 9 / 10], na[na.size() * 99 / 100], na.back());
     }
   } else {
-    launch_classic();
+    launch_k_score(ctx, ctx->stream, grid, A, C, has_var, single);
     MD_CUDA(cudaEventRecord(ctx->ev[7], ctx->stream));
   }
   unsigned long long h_stat[2] = {0, 0};
@@ -1595,22 +1522,5 @@ void score_run_dev(md_ctx* ctx, const SpectraDev& S, uint64_t n_peaks, const md_
   { float ms = 0; cudaEventElapsedTime(&ms, ctx->ev[6], ctx->ev[7]); ctx->acc_ms_kscore += ms; ctx->acc_pairs += h_stat[0]; ctx->acc_score_bytes += h_stat[1]; }
   { float ms = 0; if (cudaEventElapsedTime(&ms, ctx->ev_side0, ctx->ev_side1) == cudaSuccess) ctx->acc_ms_prepare += ms; else cudaGetLastError(); }
   ctx->acc_left += pipe ? n_left : 0u; ctx->acc_pipelined = pipe ? 1u : 0u;
-  if (timing && pipe) {
-    unsigned long long t[12];
-    MD_CUDA(cudaMemcpy(t, W.stat64.p + 8, sizeof(t), cudaMemcpyDeviceToHost));
-    fprintf(stderr, "[md_score_timing] scorer warp 0 waits by cause, cycles/CTA: slot still in use=%.0f, loader preparing=%.0f, copies in flight=%.0f, ring full=%.0f\n",
-            (double)t[8] / grid, (double)t[9] / grid, (double)t[10] / grid, (double)t[11] / grid);
-    fprintf(stderr, "[md_score_timing] pipelined, grid=%u: cycles/CTA loader work=%.0f wait=%.0f (ring full %.1f per CTA); scorer warp 0 wait=%.0f work=%.0f; bulk copies %.0f cycles for %.0f bytes per CTA\n", grid,
-            (double)t[0] / grid, (double)t[1] / grid, (double)t[6] / grid, (double)t[2] / grid, (double)t[3] / grid, (double)t[7] / grid, (double)t[4] / grid);
-  }
-  if (timing && !pipe) {
-    unsigned long long t[8];
-    MD_CUDA(cudaMemcpy(t, W.stat64.p + 8, sizeof(t), cudaMemcpyDeviceToHost));
-    double tot = 0; for (int k = 0; k < 7; k++) tot += (double)t[k];
-    static const char* names[7] = {"stage+blocks", "sort", "map+zero", "differences", "score", "topk", "scan"};
-    fprintf(stderr, "[md_score_timing] grid=%u", grid);
-    for (int k = 0; k < 7; k++) fprintf(stderr, " %s=%.1f%%", names[k], 100.0 * (double)t[k] / tot);
-    fprintf(stderr, " cycles/CTA=%.0f\n", tot / grid);
-  }
   MD_REQUIRE(!h_flag[1], MD_ERR_UNSUPPORTED, "a spectrum needs more than 2^26 fragment bins or has more than 2^24 candidates");
 }
