@@ -172,7 +172,13 @@ MD_API int md_index_export(md_ctx* ctx, uint64_t begin, uint64_t count, uint64_t
  *    vectors (k_a over the variable letters in alphabetical order, sum <= max_variable_mods, ascending as mixed-radix
  *    numbers with the last letter fastest), then ascending fixed-modification weight (ties: index order), then
  *    placements with the last letter fastest, each letter's subsets in NChooseK order (utility/combinations/n_choose_k.rs:12-49).
- * Changing the mode invalidates the index (md_index_build again). */
+ * Changing the mode invalidates the index (md_index_build again).
+ * Limits of the CUDA lookup; each returns MD_ERR_UNSUPPORTED from md_candidates / md_identify*, the oracle has none:
+ *  MD_VARMOD_REFERENCE: 2^22 subsets tried for one (spectrum, peptide): sum over n <= max_variable_mods of
+ *    C(d, n), d = the peptide's residues of variable letters, when no smaller placement lands in the window.
+ *  MD_VARMOD_EXPANDED: at most 6 variable letters (a letter whose fixed modification holds the variable slot does not
+ *    count), at most 96 count vectors (C(max_variable_mods + letters, letters)), and at most 2^20 - 1 placements
+ *    (prod_a C(count_a, k_a)) of one peptide for one count vector. */
 typedef enum md_varmod_mode { MD_VARMOD_REFERENCE = 0, MD_VARMOD_EXPANDED = 1 } md_varmod_mode;
 MD_API int md_set_variable_mode(md_ctx* ctx, int mode);
 
