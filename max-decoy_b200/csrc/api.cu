@@ -194,6 +194,7 @@ int md_create(const md_config* cfg, md_ctx** out) {
     MD_CUDA(cudaEventCreateWithFlags(&c->ev_prep, cudaEventDisableTiming));
     MD_CUDA(cudaEventCreate(&c->ev_side0)); MD_CUDA(cudaEventCreate(&c->ev_side1));
     for (auto& ev : c->ev) MD_CUDA(cudaEventCreate(&ev));
+    if (c->trace) for (auto& ev : c->ev_trace) MD_CUDA(cudaEventCreate(&ev));
     *out = c;
     return MD_OK;
   } catch (const MdError& e) {
@@ -213,6 +214,7 @@ void md_destroy(md_ctx* ctx) {
   if (ctx->ev_side1) cudaEventDestroy(ctx->ev_side1);
   comm_release(ctx);
   for (auto& ev : ctx->ev) if (ev) cudaEventDestroy(ev);
+  for (auto& ev : ctx->ev_trace) if (ev) cudaEventDestroy(ev);
   cudaStream_t s = ctx->stream;
   delete ctx;  // frees the device buffers
   if (s) cudaStreamDestroy(s);

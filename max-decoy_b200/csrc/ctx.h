@@ -75,6 +75,7 @@ struct IdentifyWorkspace {
   DevBuf<uint64_t> t_size; DevBuf<int16_t> t_K; DevBuf<uint32_t> t_flag, t_pos; DevBuf<int> t_ovf, t_unsorted;
   DevBuf<uint32_t> t_list, t_off, t_base, t_queue, t_blk;
   DevBuf<uint4> t_grown; DevBuf<uint8_t> t_route; DevBuf<uint32_t> t_narrow, t_wide;   // decoy rounds: grown attempts (32 B each), repair-pass flags and lists
+  DevBuf<uint4> t_start;             // decoy rounds: the repair passes' start state of each grown attempt (64 B each)
   DevBuf<md_precursor> t_win;        // MD_VARMOD_EXPANDED: shifted windows, one per (spectrum, count vector)
   // exhaustive mode
   DevBuf<int32_t> ex_comp; DevBuf<uint64_t> ex_cum; DevBuf<uint32_t> ex_ncomp;
@@ -97,6 +98,7 @@ struct md_ctx {
   cudaStream_t stream2 = nullptr;          // side stream: work that depends on the spectra alone runs beside the decoy generation
   cudaEvent_t ev_fork = nullptr, ev_prep = nullptr, ev_side0 = nullptr, ev_side1 = nullptr;   // (ev_side*: timing of the side stream's work)
   cudaEvent_t ev[8] = {};
+  cudaEvent_t ev_trace[6] = {};   // MD_TRACE only: per-kernel times of a decoy round
   // modifications
   bool mods_set = false;
   ModTables mods;          // host copy (passed to kernels by value)

@@ -66,15 +66,27 @@ struct TSeq {  // a lane's working sequence in shared memory (alphabet indices),
   __device__ __forceinline__ uint8_t& at(uint32_t i) const { return base[i * kThreads]; }
   __device__ __forceinline__ uint32_t get(uint32_t i) const { return base[i * kThreads]; }
 };
-// The same through an explicit 32-bit shared-memory address (k_decoy_random: every access is one IMAD + LDS/STS; through the
-// generic pointer the compiler rebuilt the shared window's address in front of each).  All accesses are volatile asm: ordered
-// among themselves, invisible to the compiler's alias analysis -- the array must not be touched through C++ pointers as well.
+// k_decoy_random's sequences, word-interleaved: one 32-bit word holds four consecutive positions of one lane, position i of
+// lane l at byte ((i >> 2) * kThreads + l) * 4 + (i & 3).  Lanes never share a bank whatever position each accesses (the
+// transposed byte layout put lanes 4k..4k+3 in one bank), and the sequence moves to and from its row (alphabet indices,
+// four positions per little-endian word) in whole words.  Accessed through an explicit 32-bit shared-memory address `a` =
+// array + 4 * lane; the byte offset of position i is IMAD + LOP3: i * 129 = (i << 7) | i for i < 128, and the mask keeps
+// (i >> 2) << 9 and i & 3; it is added to `a`, not OR-ed, as the array's shared address need not be a multiple of its size.
+// All accesses are volatile asm: ordered among themselves, invisible to the compiler's alias analysis -- the array must not
+// be touched through C++ pointers as well.
+constexpr uint32_t kSeqWordStride = kThreads * 4u;     // bytes between the words of one lane
+static_assert(kSeqWordStride == 512u, "SSeq::addr builds (i >> 2) * kSeqWordStride by masking i * 129");
 struct SSeq {
   uint32_t a;
+  __device__ __forceinline__ uint32_t addr(uint32_t i) const { return ((i * 129u) & ~0x1FCu) + a; }
   __device__ __forceinline__ uint32_t get(uint32_t i) const {
-    uint32_t v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a + i * kThreads)); return v;
+    uint32_t v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(addr(i))); return v;
   }
-  __device__ __forceinline__ void set(uint32_t i, uint32_t v) const { asm volatile("st.shared.u8 [%0], %1;" ::"r"(a + i * kThreads), "r"(v)); }
+  __device__ __forceinline__ void set(uint32_t i, uint32_t v) const { asm volatile("st.shared.u8 [%0], %1;" ::"r"(addr(i)), "r"(v)); }
+  __device__ __forceinline__ uint32_t get_word(uint32_t k) const {   // positions 4k .. 4k+3
+    uint32_t v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a + k * kSeqWordStride)); return v;
+  }
+  __device__ __forceinline__ void set_word(uint32_t k, uint32_t v) const { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a + k * kSeqWordStride), "r"(v)); }
 };
 template <class SeqT>
 struct SeqCode {  // view as residue codes for md_try_variable
@@ -148,10 +160,10 @@ struct RngRing {
   uint32_t addr;                 // shared-memory address of the lane's kRing words, stride kThreads (accessed through volatile asm only)
   uint32_t k0, k1, c0, c1, c2;   // key, next block, attempt, spectrum
   uint32_t head, count;
-  // continue the stream of (seed, spectrum_id, attempt) at word w: block w / 4, its first w % 4 words skipped
-  __device__ __forceinline__ void resume(uint64_t seed, uint32_t spectrum_id, uint32_t attempt, uint32_t w) {
-    k0 = (uint32_t)seed; k1 = (uint32_t)(seed >> 32); c0 = w >> 2; c1 = attempt; c2 = spectrum_id; head = 0; count = 0;
-    produce();
+  // continue the stream of (seed, spectrum_id, attempt) at word w, given block w / 4 (its first w % 4 words are skipped)
+  __device__ __forceinline__ void resume(uint64_t seed, uint32_t spectrum_id, uint32_t attempt, uint32_t w, uint4 block) {
+    k0 = (uint32_t)seed; k1 = (uint32_t)(seed >> 32); c0 = (w >> 2) + 1u; c1 = attempt; c2 = spectrum_id;
+    put(0, block.x); put(1, block.y); put(2, block.z); put(3, block.w);
     head = w & 3u; count = 4u - (w & 3u);
   }
   __device__ __forceinline__ void put(uint32_t t, uint32_t v) const { asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr + (t & (kRing - 1)) * (kThreads * 4u)), "r"(v)); }
@@ -173,7 +185,7 @@ struct RngRing {
 #endif
 constexpr uint32_t kRngPeriod = MD_RNG_PERIOD;
 #ifndef MD_REFILL_MIN
-#define MD_REFILL_MIN 6
+#define MD_REFILL_MIN 3
 #endif
 constexpr int kRefillMin = MD_REFILL_MIN;   // free lanes of a warp that trigger a refill
 
@@ -274,16 +286,27 @@ struct __align__(16) GrownAttempt {
   int32_t d, dlo; uint32_t span, L;
   uint32_t spectrum_id, attempt; int64_t P;
 };
+// The rest of a grown attempt's start state in k_decoy_random, also written by k_decoy_grow, so that a lane's refill is
+// word copies and straight-line logic instead of a walk over the sequence and a Philox block: the alphabet indices as five
+// bit planes of the position masks (bit i of plane k = bit k of the letter at position i; low halves first, so that the
+// narrow pass reads the first 48 bytes only), the letter set, and Philox block L / 4 of the attempt's stream, where the
+// repair continues at word L.  Written and read as four uint4.
+struct __align__(16) StartState {
+  uint32_t plane_lo[5], present, block[4];
+  uint32_t plane_hi[5], pad;
+};
+static_assert(sizeof(StartState) == 64, "four uint4");
 
 // Grow phase of REFERENCE_RANDOM (decoy_generator.rs:142-159), one thread per work item of the round: uniform letters until the
 // weight exceeds the upper limit.  A sequence longer than 60 residues (VARCHAR(60) would reject it) is a failure (len = 0) here;
 // every other attempt is flagged for the repair pass of its length -- 32-bit position masks up to `narrow_max` residues, 64-bit
 // ones above -- and k_decoy_random continues its RNG stream at word L.  The sequence goes to the row as alphabet indices in
-// 16-byte stores (the finished words of a chunk wait in registers), not byte by byte.
+// 16-byte stores (the finished words of a chunk wait in registers), not byte by byte; its bit planes, letter set and the
+// Philox block the repair resumes with go to the attempt's StartState.
 constexpr int kGrowThreads = 256;
 __global__ void __launch_bounds__(kGrowThreads) k_decoy_grow(const RandomArgs A, const __grid_constant__ DecoyTables T, AttemptOut O,
-                                                             GrownAttempt* __restrict__ grown, uint8_t* __restrict__ to_narrow,
-                                                             uint8_t* __restrict__ to_wide, uint32_t narrow_max) {
+                                                             GrownAttempt* __restrict__ grown, StartState* __restrict__ start,
+                                                             uint8_t* __restrict__ to_narrow, uint8_t* __restrict__ to_wide, uint32_t narrow_max) {
   __shared__ int32_t s_m[32];
   if (threadIdx.x < 32) s_m[threadIdx.x] = (int32_t)T.mprime[threadIdx.x];
   __syncthreads();
@@ -296,9 +319,12 @@ __global__ void __launch_bounds__(kGrowThreads) k_decoy_grow(const RandomArgs A,
   int64_t w = MD_WATER_UDA;
   uint32_t L = 0, b = 0, word = 0;
   uint32_t w0 = 0, w1 = 0, w2 = 0;   // the finished words of the current 16-byte chunk, the newest in w2
+  uint64_t plane[5] = {0, 0, 0, 0, 0};
+  uint32_t present = 0;
+  uint4 r;
   bool dead = false;
   for (;; b++) {   // Philox block b = words 4b .. 4b+3 = residues 4b .. 4b+3 = the b-th 32-bit word of the row
-    const uint4 r = philox_block(b, attempt, pr.spectrum_id, (uint32_t)A.seed, (uint32_t)(A.seed >> 32));
+    r = philox_block(b, attempt, pr.spectrum_id, (uint32_t)A.seed, (uint32_t)(A.seed >> 32));
     const uint32_t rw[4] = {r.x, r.y, r.z, r.w};
     bool done = false;
     word = 0;
@@ -309,11 +335,15 @@ __global__ void __launch_bounds__(kGrowThreads) k_decoy_grow(const RandomArgs A,
         if (L >= MD_MAX_PEPTIDE_LEN) { dead = true; done = true; }
         else {
           word |= a << (8 * j); L++;
+          present |= 1u << a;
           w += s_m[a];
           done = w > pr.hi;
         }
       }
     }
+    // bit k of the word's four letters -> bits 4b .. 4b+3 of plane k (the multiply gathers bit 0 of each byte into bits 24..27)
+#pragma unroll
+    for (int k = 0; k < 5; k++) plane[k] |= (uint64_t)((((word >> k) & 0x01010101u) * 0x01020408u) >> 24) << (4u * b);
     if (done) break;
     if ((b & 3u) == 3u) row[b >> 2] = make_uint4(w0, w1, w2, word);
     else { w0 = w1; w1 = w2; w2 = word; }
@@ -326,12 +356,19 @@ __global__ void __launch_bounds__(kGrowThreads) k_decoy_grow(const RandomArgs A,
   for (uint32_t k = b & 3u; k < 3u; k++) { w0 = w1; w1 = w2; w2 = word; word = 0; }   // the last chunk: its words in front
   row[b >> 2] = make_uint4(w0, w1, w2, word);
   grown[wi] = GrownAttempt{(int32_t)dd, (int32_t)dl, (uint32_t)sp, L, pr.spectrum_id, attempt, pr.mass};
+  // the repair continues at word L: block b unless the last letter took its last word (L == 4b + 4)
+  if ((L >> 2) != b) r = philox_block(L >> 2, attempt, pr.spectrum_id, (uint32_t)A.seed, (uint32_t)(A.seed >> 32));
+  uint4* st = reinterpret_cast<uint4*>(start + wi);
+  st[0] = make_uint4((uint32_t)plane[0], (uint32_t)plane[1], (uint32_t)plane[2], (uint32_t)plane[3]);
+  st[1] = make_uint4((uint32_t)plane[4], present, r.x, r.y);
+  st[2] = make_uint4(r.z, r.w, (uint32_t)(plane[0] >> 32), (uint32_t)(plane[1] >> 32));
+  st[3] = make_uint4((uint32_t)(plane[2] >> 32), (uint32_t)(plane[3] >> 32), (uint32_t)(plane[4] >> 32), 0u);
 }
 
 struct RepairArgs {
   const uint32_t* items; const uint32_t* n_items;   // the attempts of this pass (k_decoy_grow's narrow or wide list) and their count
   uint32_t* queue;                                   // work counter of this launch
-  GrownAttempt* grown;
+  GrownAttempt* grown; const StartState* start;
   uint64_t seed; int* overflow;
 };
 
@@ -347,15 +384,17 @@ struct RepairArgs {
 // leaves its alphabet-index sequence in the row, its mask, its length and its final d; k_decoy_finish does the rest.
 // VMODE: 0 = no variable modification can apply, 1 = one variable letter without a fixed modification (its positions are
 // tracked, try_variable_modifications needs no walk over the sequence), 2 = anything else (generic enumeration).
+// (The wide pass is bounded to 6 CTAs/SM, all that its shared memory allows: unbounded, its 64-bit refill took 88 registers.)
 template <int VMODE, class MaskT>
-__global__ void __launch_bounds__(kThreads, sizeof(MaskT) == 4 ? (VMODE < 2 ? 10 : 8) : 1) k_decoy_random(const RepairArgs A, const __grid_constant__ ModTables M, const __grid_constant__ DecoyTables T,
+__global__ void __launch_bounds__(kThreads, sizeof(MaskT) == 4 ? (VMODE < 2 ? 10 : 8) : 6) k_decoy_random(const RepairArgs A, const __grid_constant__ ModTables M, const __grid_constant__ DecoyTables T,
                                                            AttemptOut O) {
   using MO = MaskOps<MaskT>;
   constexpr uint32_t kBits = MO::bits;
   constexpr bool kNarrow = kBits < MD_MAX_PEPTIDE_LEN;
   constexpr uint32_t kRows = kNarrow ? kBits : MD_MAX_PEPTIDE_LEN;
   constexpr uint32_t kAbove = tabs::kAboveOfs;       // offset of the d < 0 tables
-  __shared__ uint8_t sseq[kRows * kThreads];
+  constexpr uint32_t kSeqWords = (kRows + 15u) / 16u * 4u;   // whole 16-byte chunks of the row per lane (the refill copies chunks)
+  __shared__ __align__(16) uint8_t sseq[kSeqWords * kSeqWordStride];
   __shared__ uint32_t s_rng[kRing * kThreads];
   __shared__ MaskT s_pm[MD_ALPHABET_SIZE * kThreads];   // per lane and letter: the positions holding that letter
   __shared__ __align__(16) uint8_t s_tab[tabs::bytes];   // the lookup tables (namespace tabs)
@@ -377,7 +416,7 @@ __global__ void __launch_bounds__(kThreads, sizeof(MaskT) == 4 ? (VMODE < 2 ? 10
   uint32_t tb;    // the block's shared-memory address (made opaque: it is to stay in a register, not to be rebuilt per lookup)
   asm volatile("mov.u32 %0, %1;" : "=r"(tb) : "r"((uint32_t)__cvta_generic_to_shared(s_tab)) : "memory");   // (the tables' stores above stay in front of it)
   SSeq seq;
-  asm volatile("mov.u32 %0, %1;" : "=r"(seq.a) : "r"((uint32_t)__cvta_generic_to_shared(sseq) + threadIdx.x));
+  asm volatile("mov.u32 %0, %1;" : "=r"(seq.a) : "r"((uint32_t)__cvta_generic_to_shared(sseq) + 4u * threadIdx.x));
   const uint32_t gap_shift = T.gap_shift, nn_shift = T.nn_shift;
   const int32_t nn_lo = T.nn_lo, nn_hi = T.nn_hi;
   const int va = VMODE == 1 ? md_alpha_of_code((uint32_t)M.var_simple_code) : -1;
@@ -408,19 +447,12 @@ __global__ void __launch_bounds__(kThreads, sizeof(MaskT) == 4 ? (VMODE < 2 ? 10
     if (__popc(busy_m) <= 32 - kRefillMin) free_m = __ballot_sync(0xffffffffu, !busy && (!drained || pending));
     if (free_m && (__popc(free_m) >= kRefillMin || busy_m == 0)) {
       if (!busy && pending) {
-        if (pending == 1) {   // the final sequence (alphabet indices) back into the row, 16 bytes at a time
+        if (pending == 1) {   // the final sequence (alphabet indices) back into the row, 16 bytes at a time (k_decoy_finish
+                              // reads the positions < L only)
           uint4* row = reinterpret_cast<uint4*>(O.rows + (size_t)wi * MD_DECOY_ROW);
-#pragma unroll 1
-          for (uint32_t c = 0; 16u * c < L; c++) {
-            uint32_t wd[4];
 #pragma unroll
-            for (uint32_t j = 0; j < 16; j++) {
-              const uint32_t i = 16u * c + j;
-              const uint32_t a = i < L ? seq.get(i) : 0u;
-              wd[j >> 2] = (j & 3) ? wd[j >> 2] | a << (8 * (j & 3)) : a;
-            }
-            row[c] = make_uint4(wd[0], wd[1], wd[2], wd[3]);
-          }
+          for (uint32_t c = 0; c < kSeqWords / 4u; c++)
+            if (16u * c < L) row[c] = make_uint4(seq.get_word(4u * c), seq.get_word(4u * c + 1u), seq.get_word(4u * c + 2u), seq.get_word(4u * c + 3u));
           O.mask[wi] = (uint64_t)mask; A.grown[wi].d = d;
         }
         O.len[wi] = pending == 1 ? (uint8_t)L : 0;
@@ -432,29 +464,39 @@ __global__ void __launch_bounds__(kThreads, sizeof(MaskT) == 4 ? (VMODE < 2 ? 10
         else {
           wi = A.items[q];
           const GrownAttempt* g = A.grown + wi;
+          const uint4* st = reinterpret_cast<const uint4*>(A.start + wi);
+          const uint4* row = reinterpret_cast<const uint4*>(O.rows + (size_t)wi * MD_DECOY_ROW);
           L = g->L; d = g->d; dlo = g->dlo; span = g->span;
           if (VMODE == 2) P = g->P;
-          rng.resume(A.seed, g->spectrum_id, g->attempt, L);   // the grow phase drew L words
-          // the grown sequence into the lane's shared-memory state: letters, per-letter position masks, variable positions
-          mask = 0; vpos = 0; present = 0;
-          for (int a = 0; a < MD_ALPHABET_SIZE; a++) MO::st(pm_a + a * kPmStride, (MaskT)0);
-          const uint4* row = reinterpret_cast<const uint4*>(O.rows + (size_t)wi * MD_DECOY_ROW);
-#pragma unroll 1
-          for (uint32_t c = 0; 16u * c < L; c++) {
-            const uint4 v = row[c];
-            const uint32_t wd[4] = {v.x, v.y, v.z, v.w};
+          const uint4 s0 = st[0], s1 = st[1], s2 = st[2];
+          MaskT pl[5] = {s0.x, s0.y, s0.z, s0.w, s1.x};   // the bit planes (StartState)
+          if (!kNarrow) {
+            const uint4 s3 = st[3];
+            const uint32_t hi[5] = {s2.z, s2.w, s3.x, s3.y, s3.z};
 #pragma unroll
-            for (uint32_t j = 0; j < 16; j++) {
-              const uint32_t i = 16u * c + j;
-              if (i < L) {
-                const uint32_t a = (wd[j >> 2] >> (8 * (j & 3))) & 0xFFu;
-                if (VMODE == 1 && (int)a == va) vpos |= (MaskT)1 << i;
-                add_letter(a, i); seq.set(i, a);
-              }
-            }
+            for (int k = 0; k < 5; k++) pl[k] |= (MaskT)hi[k] << (kBits / 2);
           }
-          busy = true; tries = 0; pos = 0;
+          present = s1.y;
+          rng.resume(A.seed, g->spectrum_id, g->attempt, L, make_uint4(s1.z, s1.w, s2.x, s2.y));   // the grow phase drew L words
           lmask = L >= kBits ? ~(MaskT)0 : (((MaskT)1 << L) - 1);
+          // the per-letter position masks: the positions whose letter has the bits of a, from the planes (a is a constant of
+          // the unrolled loop; positions >= L have all planes 0, so only letter 0 needs lmask)
+#pragma unroll
+          for (uint32_t a = 0; a < MD_ALPHABET_SIZE; a++) {
+            const MaskT m = ((a & 1u) ? pl[0] : ~pl[0]) & ((a & 2u) ? pl[1] : ~pl[1]) & ((a & 4u) ? pl[2] : ~pl[2]) &
+                            ((a & 8u) ? pl[3] : ~pl[3]) & ((a & 16u) ? pl[4] : ~pl[4]);
+            MO::st(pm_a + a * kPmStride, a == 0 ? m & lmask : m);
+          }
+          mask = 0;
+          if (VMODE == 1) vpos = MO::ld(pm_a + (uint32_t)va * kPmStride);
+          // the sequence, whole 16-byte chunks of the row (positions >= L are never read)
+#pragma unroll
+          for (uint32_t c = 0; c < kSeqWords / 4u; c++)
+            if (16u * c < L) {
+              const uint4 v = row[c];
+              seq.set_word(4u * c, v.x); seq.set_word(4u * c + 1u, v.y); seq.set_word(4u * c + 2u, v.z); seq.set_word(4u * c + 3u, v.w);
+            }
+          busy = true; tries = 0; pos = 0;
         }
       }
       busy_m = __ballot_sync(0xffffffffu, busy);
@@ -1131,6 +1173,7 @@ void decoys_generate_dev(md_ctx* ctx, uint32_t n, uint32_t n_per, int mode, uint
     level_begin[kRoundLevels] = (uint32_t)list.size();
     if (list.empty()) break;
     const uint32_t n_list = (uint32_t)list.size(), total = off.back();
+    bool split = false;    // ev_trace holds this round's per-kernel times
     W.att_rows.need((size_t)total * MD_DECOY_ROW + 64); W.att_len.need(total + 1); W.att_mask.need(total + 1); W.att_w.need(total + 1); W.att_hash.need(total + 1);
     AttemptOut O{W.att_rows.p, W.att_len.p, W.att_mask.p, W.att_w.p, W.att_hash.p};
     MD_CUDA(cudaMemcpyAsync(d_list.p, list.data(), n_list * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
@@ -1160,18 +1203,29 @@ void decoys_generate_dev(md_ctx* ctx, uint32_t n, uint32_t n_per, int mode, uint
         // masks; finish the hits.  The two lists keep the work-item order (spectra by mass: neighbouring lanes repair
         // sequences of similar length).
         const size_t tpad = ((size_t)total + 15) & ~(size_t)15;
-        W.t_grown.need(2 * (size_t)total + 2); W.t_route.need(2 * tpad); W.t_narrow.need((size_t)total + 1); W.t_wide.need((size_t)total + 1);
+        W.t_grown.need(2 * (size_t)total + 2); W.t_start.need(4 * (size_t)total + 4); W.t_route.need(2 * tpad); W.t_narrow.need((size_t)total + 1);
+        W.t_wide.need((size_t)total + 1);
         GrownAttempt* grown = reinterpret_cast<GrownAttempt*>(W.t_grown.p);
+        StartState* start = reinterpret_cast<StartState*>(W.t_start.p);
         uint8_t* to_narrow = W.t_route.p; uint8_t* to_wide = W.t_route.p + tpad;
+        // (MD_TRACE: an event behind each step, printed with the round's line)
+        auto trace_ev = [&](int i) { if (ctx->trace) MD_CUDA(cudaEventRecord(ctx->ev_trace[i], ctx->stream)); };
         MD_CUDA(cudaMemsetAsync(d_queue.p, 0, 4 * sizeof(uint32_t), ctx->stream));
-        MD_LAUNCH(ctx, k_decoy_grow, blocks(total, kGrowThreads), kGrowThreads, 0, RA, T, O, grown, to_narrow, to_wide, wide_only ? 0u : 32u);
+        trace_ev(0);
+        MD_LAUNCH(ctx, k_decoy_grow, blocks(total, kGrowThreads), kGrowThreads, 0, RA, T, O, grown, start, to_narrow, to_wide, wide_only ? 0u : 32u);
+        trace_ev(1);
         cubx_select_flagged_index(ctx, to_narrow, W.t_narrow.p, d_queue.p + 1, total);
         cubx_select_flagged_index(ctx, to_wide, W.t_wide.p, d_queue.p + 3, total);
-        RepairArgs R{W.t_narrow.p, d_queue.p + 1, d_queue.p, grown, seed, d_ovf.p};
+        trace_ev(2);
+        RepairArgs R{W.t_narrow.p, d_queue.p + 1, d_queue.p, grown, start, seed, d_ovf.p};
         if (!wide_only) launch_random<uint32_t>(ctx, vmode, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * (uint32_t)occ_narrow), R, T, O);
-        R = RepairArgs{W.t_wide.p, d_queue.p + 3, d_queue.p + 2, grown, seed, d_ovf.p};
+        trace_ev(3);
+        R = RepairArgs{W.t_wide.p, d_queue.p + 3, d_queue.p + 2, grown, start, seed, d_ovf.p};
         launch_random<uint64_t>(ctx, vmode, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * (uint32_t)occ_wide), R, T, O);
+        trace_ev(4);
         MD_LAUNCH(ctx, k_decoy_finish, blocks(total, 256), 256, 0, total, T, O, grown, PV);
+        trace_ev(5);
+        split = ctx->trace;
       }
     } else {
       MD_LAUNCH(ctx, k_decoy_permute, blocks(total, kThreads), kThreads, 0, W.prec.p, d_list.p, d_off.p, d_base.p, n_list, total, seed, T, W.cand_off.p,
@@ -1203,7 +1257,12 @@ void decoys_generate_dev(md_ctx* ctx, uint32_t n, uint32_t n_per, int mode, uint
     ctx->mark("  select");
     for (uint32_t i = 0; i < n_list; i++) used[list[i]] += off[i + 1] - off[i];
     { float ms = 0; cudaEventElapsedTime(&ms, ctx->ev[4], ctx->ev[5]); ctx->acc_ms_kdecoy += ms; ctx->acc_attempts += total;
-      if (ctx->trace) fprintf(stderr, "[md_trace]   decoy round %d: spectra=%u attempts=%u kernel=%.3f ms\n", round, n_list, total, ms); }
+      if (ctx->trace) fprintf(stderr, "[md_trace]   decoy round %d: spectra=%u attempts=%u kernel=%.3f ms\n", round, n_list, total, ms);
+      if (split) {
+        float t[5];
+        for (int i = 0; i < 5; i++) MD_CUDA(cudaEventElapsedTime(&t[i], ctx->ev_trace[i], ctx->ev_trace[i + 1]));
+        fprintf(stderr, "[md_trace]   decoy round %d kernels: grow=%.3f lists=%.3f narrow=%.3f wide=%.3f finish=%.3f ms\n", round, t[0], t[1], t[2], t[3], t[4]);
+      } }
   }
   const int ovf = d2h_scalar(ctx, d_ovf.p);
   MD_REQUIRE(ovf != 3, MD_ERR_DEVICE, "decoy generation: internal error (substitution filter disagrees with the mass search)");
