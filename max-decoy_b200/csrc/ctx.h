@@ -52,14 +52,14 @@ struct IdentifyWorkspace {
   DevBuf<uint64_t> flat_off;         // prefix of range sizes (n+1)
   DevBuf<uint64_t> cand_off;         // CSR of accepted targets (n+1)
   // per index entry in the flattened ranges
-  DevBuf<uint8_t> flag; DevBuf<uint64_t> emask; DevBuf<int64_t> ew; DevBuf<uint64_t> epos;
+  DevBuf<uint64_t> emask; DevBuf<int64_t> ew;
   // accepted targets
   DevBuf<uint64_t> cand_desc; DevBuf<uint64_t> cand_mask; DevBuf<int64_t> cand_w; DevBuf<uint32_t> cand_pep;
   // decoy attempts (one slot per attempt of the current round) and accepted decoys (n_per slots per spectrum)
   DevBuf<uint8_t> att_rows; DevBuf<uint8_t> att_len; DevBuf<uint64_t> att_mask; DevBuf<int64_t> att_w; DevBuf<uint64_t> att_hash;
   DevBuf<uint8_t> dec_rows; DevBuf<uint8_t> dec_len; DevBuf<uint64_t> dec_mask; DevBuf<int64_t> dec_w; DevBuf<uint64_t> dec_hash;
-  DevBuf<uint32_t> dec_attempt; DevBuf<uint32_t> dec_count; DevBuf<uint32_t> att_base; DevBuf<uint32_t> att_limit;
-  DevBuf<uint32_t> work_list; DevBuf<uint32_t> counters; DevBuf<unsigned long long> stat64;
+  DevBuf<uint32_t> dec_attempt; DevBuf<uint32_t> dec_count;
+  DevBuf<uint32_t> counters; DevBuf<unsigned long long> stat64;
   // binned spectra
   DevBuf<uint16_t> gmap; DevBuf<uint32_t> gbits;   // per-CTA block maps in HBM (tables beyond the shared-memory map)
   DevBuf<int32_t> pk_bin; DevBuf<int32_t> pk_yq; DevBuf<uint32_t> pk_count; DevBuf<int32_t> pk_hbin;
@@ -77,17 +77,11 @@ struct IdentifyWorkspace {
   DevBuf<uint4> t_grown; DevBuf<uint8_t> t_route; DevBuf<uint32_t> t_narrow, t_wide;   // decoy rounds: grown attempts (32 B each), repair-pass flags and lists
   DevBuf<uint4> t_start;             // decoy rounds: the repair passes' start state of each grown attempt (64 B each)
   DevBuf<md_precursor> t_win;        // MD_VARMOD_EXPANDED: shifted windows, one per (spectrum, count vector)
-  // exhaustive mode
-  DevBuf<int32_t> ex_comp; DevBuf<uint64_t> ex_cum; DevBuf<uint32_t> ex_ncomp;
 };
 
-struct LastDecoys {
+struct LastDecoys {   // the batch of the last identify call with keep_decoys: its decoys stay in ws.dec_*
   bool have = false;
   uint32_t n_spectra = 0, n_per = 0;
-  std::vector<uint8_t> rows, len;
-  std::vector<uint64_t> mask;
-  std::vector<int64_t> w;
-  std::vector<uint32_t> attempt, count;
 };
 
 struct md_ctx {

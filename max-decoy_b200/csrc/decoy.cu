@@ -21,7 +21,7 @@ inline uint32_t blocks(uint64_t n, uint32_t bs = 256) { return (uint32_t)((n + b
 
 constexpr int kThreads = 128;          // lanes per CTA of the attempt kernels
 // MD_ROUND_ATTEMPTS and MD_SELECT_SMEM_MAX (test builds only) shrink the list entries and the hash selection's shared-memory
-// budget, so that small inputs run several levels per round and reach k_decoy_select_n2
+// budget, so that small inputs run several levels per round and reach k_decoy_select's exact route
 #ifndef MD_ROUND_ATTEMPTS
 #define MD_ROUND_ATTEMPTS 4096
 #endif
@@ -36,12 +36,7 @@ constexpr int kRoundLevels = 4;          // list entries one spectrum can have i
 constexpr uint32_t kGapTab = 512, kNnTab = 1024;
 struct DecoyTables {
   int64_t mprime[32];      // residue mass + fixed delta, by alphabet index (0..20)
-  int64_t sorted_m[32];    // mprime sorted ascending (ties by alphabet index), padded with INT64_MAX
-  uint8_t sorted_a[32];    // alphabet index at each sorted position
-  uint8_t run_min_a[32];   // lowest alphabet index among entries of equal mass
   uint8_t code_of_a[32];   // residue code of alphabet index
-  uint8_t has_var_a[32];
-  uint8_t has_fix_a[32];
   int64_t var_a[32];
   // improving-substitution filter: letter a has a substitution that strictly reduces |d| iff its gap to the next lighter
   // (d > 0) / heavier (d < 0) distinct mass is < 2|d|.  Gaps sorted ascending + the letter set of every prefix.
@@ -120,16 +115,11 @@ __device__ void store_attempt(const AttemptOut& O, uint64_t slot, const SeqT& se
   O.len[slot] = (uint8_t)L; O.mask[slot] = mask; O.w[slot] = w; O.hash[slot] = h;
 }
 
-// work item -> (list entry, attempt ordinal) by binary search on the round's prefix of attempt counts
-// the same with a coarse table: blk[b] = entry of work item b << kBlkLog (the search runs between two neighbouring table values)
+// work item -> (list entry, attempt ordinal) by binary search on the round's prefix of attempt counts, narrowed by a coarse
+// table: blk[b] = entry of work item b << kBlkLog (the search runs between two neighbouring table values)
 constexpr uint32_t kBlkLog = 10;
 __device__ __forceinline__ uint32_t find_entry_coarse(const uint32_t* __restrict__ att_off, const uint32_t* __restrict__ blk, uint32_t w) {
   uint32_t lo = blk[w >> kBlkLog], hi = blk[(w >> kBlkLog) + 1] + 1u;   // att_off[lo] <= w < att_off[hi]
-  while (hi - lo > 1) { uint32_t mid = (lo + hi) >> 1; if (att_off[mid] <= w) lo = mid; else hi = mid; }
-  return lo;
-}
-__device__ __forceinline__ uint32_t find_entry(const uint32_t* __restrict__ att_off, uint32_t n_list, uint32_t w) {
-  uint32_t lo = 0, hi = n_list;
   while (hi - lo > 1) { uint32_t mid = (lo + hi) >> 1; if (att_off[mid] <= w) lo = mid; else hi = mid; }
   return lo;
 }
@@ -275,7 +265,7 @@ template <uint32_t OFF> __device__ __forceinline__ uint32_t tab_u8(uint32_t addr
 struct RandomArgs {   // the work items of a round: list entries (spectrum, attempt ordinals) and their prefix of attempt counts
   const md_precursor* prec; const uint32_t* list; const uint32_t* att_off; const uint32_t* att_base;
   const uint32_t* att_blk;              // coarse index into att_off (find_entry_coarse)
-  uint32_t n_list, total;
+  uint32_t total;
   uint64_t seed; int* overflow;
 };
 
@@ -648,7 +638,7 @@ __global__ void __launch_bounds__(kThreads) k_decoy_random_terminal(const Random
   TSeq seq{sseq + threadIdx.x};
   auto fixd = [&](uint32_t a, uint32_t i, uint32_t L) -> int64_t { const uint32_t c = T.code_of_a[a]; return md_fix_applies(M, c, i, L) ? M.fix[c] : 0; };
   for (uint32_t wi = blockIdx.x * blockDim.x + threadIdx.x; wi < A.total; wi += gridDim.x * blockDim.x) {
-    const uint32_t li = find_entry(A.att_off, A.n_list, wi);
+    const uint32_t li = find_entry_coarse(A.att_off, A.att_blk, wi);
     const md_precursor pr = A.prec[A.list[li]];
     Philox4 rng; rng.init(A.seed, pr.spectrum_id, A.att_base[li] + (wi - A.att_off[li]), MD_TAG_RANDOM);
     // grow (decoy_generator.rs:142-159; push_modification, modified_peptide.rs:182-208: the residue that was last loses its
@@ -698,9 +688,7 @@ __global__ void __launch_bounds__(kThreads) k_decoy_random_terminal(const Random
 }
 
 // vary_targets (decoy_generator.rs:265-296), counter-based: attempt a shuffles target (a mod T) of the spectrum
-__global__ void __launch_bounds__(kThreads) k_decoy_permute(const md_precursor* __restrict__ prec, const uint32_t* __restrict__ list,
-                                                            const uint32_t* __restrict__ att_off, const uint32_t* __restrict__ att_base, uint32_t n_list,
-                                                            uint32_t total, uint64_t seed, const __grid_constant__ DecoyTables T,
+__global__ void __launch_bounds__(kThreads) k_decoy_permute(const RandomArgs A, const __grid_constant__ DecoyTables T,
                                                             const uint64_t* __restrict__ cand_off, const uint64_t* __restrict__ cand_desc,
                                                             const uint64_t* __restrict__ cand_mask, const int64_t* __restrict__ cand_w,
                                                             const uint8_t* __restrict__ idx_rows, AttemptOut O, PeptideView PV,
@@ -708,11 +696,11 @@ __global__ void __launch_bounds__(kThreads) k_decoy_permute(const md_precursor* 
   __shared__ uint8_t sseq[MD_MAX_PEPTIDE_LEN * kThreads];
   TSeq seq{sseq + threadIdx.x};
   const uint32_t wi = blockIdx.x * blockDim.x + threadIdx.x;
-  if (wi >= total) return;
-  const uint32_t li = find_entry(att_off, n_list, wi);
-  const uint32_t s = list[li];
-  const md_precursor pr = prec[s];
-  const uint32_t attempt = att_base[li] + (wi - att_off[li]);
+  if (wi >= A.total) return;
+  const uint32_t li = find_entry_coarse(A.att_off, A.att_blk, wi);
+  const uint32_t s = A.list[li];
+  const md_precursor pr = A.prec[s];
+  const uint32_t attempt = A.att_base[li] + (wi - A.att_off[li]);
   const uint64_t t0 = cand_off[s], nt = cand_off[s + 1] - t0;
   if (nt == 0) { O.len[wi] = 0; return; }
   const uint64_t c = t0 + attempt % nt;
@@ -734,7 +722,7 @@ __global__ void __launch_bounds__(kThreads) k_decoy_permute(const md_precursor* 
     seq.at(i) = (uint8_t)(a < 0 ? 0 : a);
   }
   if (!ok) { O.len[wi] = 0; return; }
-  Philox4 rng; rng.init(seed, pr.spectrum_id, attempt, MD_TAG_PERMUTE);
+  Philox4 rng; rng.init(A.seed, pr.spectrum_id, attempt, MD_TAG_PERMUTE);
   for (uint32_t i = L; i > 1; i--) {
     uint32_t j = rng.below(i);
     uint8_t a = seq.at(i - 1); seq.at(i - 1) = seq.at(j); seq.at(j) = a;
@@ -749,26 +737,29 @@ __global__ void __launch_bounds__(kThreads) k_decoy_permute(const md_precursor* 
 
 // One CTA per listed spectrum: keep the successes of this round that are new (not equal to an accepted decoy or to an
 // earlier success), in attempt order, until the spectrum has n_per decoys (HashSet<Decoy>, decoy_generator.rs:40,164).
-// Linear time: accepted decoys and successes go into a shared-memory hash set keyed by the 64-bit sequence hash, each
-// entry remembering the lowest ordinal (accepted decoys first, then attempts in order) that carried the key; a success
-// is kept iff it is that first carrier.  A success that is NOT the first carrier of its hash is compared with that carrier
-// byte for byte: equal = a duplicate (the usual case); different = two sequences share a 64-bit hash, and the CTA redoes
-// the spectrum with exact comparisons (HashSet<Decoy> compares strings, decoy_generator.rs:40,164).  The attempt hashes are
-// read from HBM once (staged in shared memory); the kept rows are copied by the whole CTA, four lanes per 64-byte row.
+// Two routes to the keep decision; the host takes the hash set when it fits shared memory (slots > 0), else the exact scan:
+// - Hash set, linear time: accepted decoys and successes go into a shared-memory hash set keyed by the 64-bit sequence hash,
+//   each entry remembering the lowest ordinal (accepted decoys first, then attempts in order) that carried the key; a success
+//   is kept iff it is that first carrier.  A success that is NOT the first carrier of its hash is compared with that carrier
+//   byte for byte: equal = a duplicate (the usual case); different = two sequences share a 64-bit hash, and the CTA redoes
+//   the spectrum with the exact scan.
+// - Exact scan, quadratic: a success is kept iff no accepted decoy and no earlier success is the same sequence (HashSet<Decoy>
+//   compares strings).  Attempts are strided across the threads: a chunk per thread would leave the last chunk's owner
+//   comparing against nearly every success.
+// The attempt hashes are read from HBM once (staged in shared memory); the kept rows are copied by the whole CTA, four lanes
+// per 64-byte row.
 __global__ void __launch_bounds__(256) k_decoy_select(const uint32_t* __restrict__ list, const uint32_t* __restrict__ att_off,
                                                       const uint32_t* __restrict__ att_base, uint32_t n_per, uint32_t slots, uint32_t max_na, AttemptOut A,
-                                                      uint64_t n_slots, uint8_t* __restrict__ dec_rows, uint8_t* __restrict__ dec_len, uint64_t* __restrict__ dec_mask,
-                                                      int64_t* __restrict__ dec_w, uint64_t* __restrict__ dec_hash, uint32_t* __restrict__ dec_attempt,
-                                                      uint32_t* __restrict__ dec_count) {
+                                                      DecoyOut D) {
   extern __shared__ __align__(16) unsigned long long s_key[];     // slots (0 = empty)
   unsigned long long* s_hash = s_key + slots;                     // max_na: hash of a success (0 -> 1), 0 = failed attempt
   uint32_t* s_ord = reinterpret_cast<uint32_t*>(s_hash + max_na); // slots
-  uint16_t* s_list = reinterpret_cast<uint16_t*>(s_ord + slots);  // max_na: kept attempts, in order
+  uint16_t* s_list = reinterpret_cast<uint16_t*>(s_ord + slots);  // max_na: kept attempts, in order (before that: the exact scan's keep flags)
   __shared__ uint32_t s_wsum[8];
   __shared__ uint32_t s_collision;
   const uint32_t li = blockIdx.x, s = list[li];
   const uint32_t a0 = att_off[li], na = att_off[li + 1] - a0;
-  const uint32_t have = dec_count[s];
+  const uint32_t have = D.count[s];
   const uint64_t dbase = (uint64_t)s * n_per;
   const uint32_t smask = slots - 1;
   const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -778,8 +769,8 @@ __global__ void __launch_bounds__(256) k_decoy_select(const uint32_t* __restrict
     const uint32_t L = A.len[a0 + a];
     const uint8_t* mine = A.rows + (uint64_t)(a0 + a) * MD_DECOY_ROW;
     if (rep < have) {
-      if (dec_len[dbase + rep] != L) return false;
-      for (uint32_t i = 0; i < L; i++) if (dec_rows[md_dec_byte(n_slots, dbase + rep, i)] != mine[i]) return false;
+      if (D.len[dbase + rep] != L) return false;
+      for (uint32_t i = 0; i < L; i++) if (D.rows[md_dec_byte(D.n_slots, dbase + rep, i)] != mine[i]) return false;
     } else {
       if (A.len[a0 + rep - have] != L) return false;
       const uint8_t* o = A.rows + (uint64_t)(a0 + rep - have) * MD_DECOY_ROW;
@@ -799,47 +790,54 @@ __global__ void __launch_bounds__(256) k_decoy_select(const uint32_t* __restrict
     s_hash[a] = L ? (h ? h : 1ULL) : 0ULL;
   }
   __syncthreads();
-  auto insert = [&](unsigned long long h, uint32_t ord) {
-    uint32_t slot = (uint32_t)h & smask;
-    for (;;) {
-      const unsigned long long prev = atomicCAS(&s_key[slot], 0ULL, h);
-      if (prev == 0ULL || prev == h) { atomicMin(&s_ord[slot], ord); return; }
-      slot = (slot + 1) & smask;
-    }
-  };
-  for (uint32_t j = tid; j < have; j += 256) { const unsigned long long h = dec_hash[dbase + j] & MD_SELECT_HASH_MASK; insert(h ? h : 1ULL, j); }
-  for (uint32_t a = tid; a < na; a += 256) { const unsigned long long h = s_hash[a]; if (h) insert(h, have + a); }
-  __syncthreads();
   // keep flags + ordered compaction: thread t owns the contiguous chunk [t*per, (t+1)*per), per <= 16
   const uint32_t per = (na + 255u) / 256u;
   const uint32_t cb = tid * per, ce = min(cb + per, na);
   uint32_t keepbits = 0, c = 0;
-  for (uint32_t a = cb; a < ce; a++) {
-    const unsigned long long h = s_hash[a];
-    bool keep = h != 0ULL;
-    if (keep) {
+  if (slots) {
+    auto insert = [&](unsigned long long h, uint32_t ord) {
       uint32_t slot = (uint32_t)h & smask;
-      while (s_key[slot] != h) slot = (slot + 1) & smask;
-      keep = s_ord[slot] == have + a;
-      if (!keep && !same_sequence(a, s_ord[slot])) s_collision = 1;    // not a duplicate after all
-    }
-    if (keep) { keepbits |= 1u << (a - cb); c++; }
-  }
-  __syncthreads();
-  if (s_collision) {   // (two sequences with one 64-bit hash: practically never) exact: kept iff no accepted decoy and no earlier success is the same sequence
-    keepbits = 0; c = 0;
+      for (;;) {
+        const unsigned long long prev = atomicCAS(&s_key[slot], 0ULL, h);
+        if (prev == 0ULL || prev == h) { atomicMin(&s_ord[slot], ord); return; }
+        slot = (slot + 1) & smask;
+      }
+    };
+    for (uint32_t j = tid; j < have; j += 256) { const unsigned long long h = D.hash[dbase + j] & MD_SELECT_HASH_MASK; insert(h ? h : 1ULL, j); }
+    for (uint32_t a = tid; a < na; a += 256) { const unsigned long long h = s_hash[a]; if (h) insert(h, have + a); }
+    __syncthreads();
     for (uint32_t a = cb; a < ce; a++) {
       const unsigned long long h = s_hash[a];
       bool keep = h != 0ULL;
-      for (uint32_t j = 0; j < have && keep; j++) { const unsigned long long hj = dec_hash[dbase + j] & MD_SELECT_HASH_MASK; if ((hj ? hj : 1ULL) == h && same_sequence(a, j)) keep = false; }
-      for (uint32_t b = 0; b < a && keep; b++) if (s_hash[b] == h && same_sequence(a, have + b)) keep = false;
+      if (keep) {
+        uint32_t slot = (uint32_t)h & smask;
+        while (s_key[slot] != h) slot = (slot + 1) & smask;
+        keep = s_ord[slot] == have + a;
+        if (!keep && !same_sequence(a, s_ord[slot])) s_collision = 1;    // not a duplicate after all
+      }
       if (keep) { keepbits |= 1u << (a - cb); c++; }
     }
+    __syncthreads();
+  }
+  if (!slots || s_collision) {   // (after a collision: two sequences with one 64-bit hash, practically never)
+    uint8_t* s_keep = reinterpret_cast<uint8_t*>(s_list);
+    for (uint32_t a = tid; a < na; a += 256) {
+      const unsigned long long h = s_hash[a];
+      bool keep = h != 0ULL;
+      // (against the accepted decoys: their hashes as stored, without the hash set's 0 -> 1)
+      const unsigned long long hr = keep ? A.hash[a0 + a] & MD_SELECT_HASH_MASK : 0ULL;
+      for (uint32_t j = 0; j < have && keep; j++) if ((D.hash[dbase + j] & MD_SELECT_HASH_MASK) == hr && same_sequence(a, j)) keep = false;
+      for (uint32_t b = 0; b < a && keep; b++) if (s_hash[b] == h && same_sequence(a, have + b)) keep = false;
+      s_keep[a] = keep;
+    }
+    __syncthreads();
+    keepbits = 0; c = 0;
+    for (uint32_t a = cb; a < ce; a++) if (s_keep[a]) { keepbits |= 1u << (a - cb); c++; }
   }
   uint32_t incl = c;
   for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((int)lane >= o) incl += t; }
   if (lane == 31) s_wsum[warp] = incl;
-  __syncthreads();
+  __syncthreads();   // (also: every keep flag is read before s_list is written)
   uint32_t before = incl - c, total = 0;
   for (uint32_t w = 0; w < 8; w++) { const uint32_t v = s_wsum[w]; if (w < warp) before += v; total += v; }
   const uint32_t room = n_per > have ? n_per - have : 0u;
@@ -862,7 +860,7 @@ __global__ void __launch_bounds__(256) k_decoy_select(const uint32_t* __restrict
 #pragma unroll
     for (int j = 0; j < 4; j++) {
       const uint32_t t = t0 + (uint32_t)j * 256u;
-      if (t < nk * 4u) *reinterpret_cast<uint4*>(dec_rows + md_dec_byte(n_slots, dbase + have + (t >> 2), (t & 3u) * 16u)) = v[j];
+      if (t < nk * 4u) *reinterpret_cast<uint4*>(D.rows + md_dec_byte(D.n_slots, dbase + have + (t >> 2), (t & 3u) * 16u)) = v[j];
     }
   }
   for (uint32_t r0 = tid; r0 < nk; r0 += 2u * 256u) {
@@ -877,99 +875,25 @@ __global__ void __launch_bounds__(256) k_decoy_select(const uint32_t* __restrict
       const uint32_t r = r0 + (uint32_t)j * 256u;
       if (r < nk) {
         const uint64_t dst = dbase + have + r;
-        dec_len[dst] = ln[j]; dec_mask[dst] = mk[j]; dec_w[dst] = wt[j]; dec_hash[dst] = hs[j];
-        dec_attempt[dst] = att_base[li] + s_list[r];
+        D.len[dst] = ln[j]; D.mask[dst] = mk[j]; D.w[dst] = wt[j]; D.hash[dst] = hs[j];
+        D.attempt[dst] = att_base[li] + s_list[r];
       }
     }
   }
-  if (tid == 0) dec_count[s] = have + nk;
+  if (tid == 0) D.count[s] = have + nk;
 }
 
-// Fallback of k_decoy_select for tables that do not fit shared memory (quadratic scan, exact sequence compare).
-// One CTA per listed spectrum: keep the successes of this round that are new (not equal to an accepted decoy or to an
-// earlier success), in attempt order, until the spectrum has n_per decoys (HashSet<Decoy>, decoy_generator.rs:40,164).
-__global__ void __launch_bounds__(256) k_decoy_select_n2(const uint32_t* __restrict__ list, const uint32_t* __restrict__ att_off,
-                                                      const uint32_t* __restrict__ att_base, uint32_t n_per, AttemptOut A, uint64_t n_slots, uint8_t* __restrict__ dec_rows,
-                                                      uint8_t* __restrict__ dec_len, uint64_t* __restrict__ dec_mask, int64_t* __restrict__ dec_w,
-                                                      uint64_t* __restrict__ dec_hash, uint32_t* __restrict__ dec_attempt, uint32_t* __restrict__ dec_count) {
-  __shared__ uint64_t s_hash[kMaxRoundAttempts];
-  __shared__ uint8_t s_keep[kMaxRoundAttempts];
-  __shared__ uint32_t s_scan[256];
-  __shared__ uint32_t s_base;
-  const uint32_t li = blockIdx.x, s = list[li];
-  const uint32_t a0 = att_off[li], na = att_off[li + 1] - a0;
-  const uint32_t have = dec_count[s];
-  const uint64_t dbase = (uint64_t)s * n_per;
-  for (uint32_t a = threadIdx.x; a < na; a += blockDim.x) s_hash[a] = A.len[a0 + a] ? A.hash[a0 + a] : 0ULL;
-  __syncthreads();
-  for (uint32_t a = threadIdx.x; a < na; a += blockDim.x) {
-    const uint32_t L = A.len[a0 + a];
-    bool keep = L != 0;
-    if (keep) {
-      const uint64_t h = s_hash[a];
-      const uint8_t* mine = A.rows + (uint64_t)(a0 + a) * MD_DECOY_ROW;
-      for (uint32_t j = 0; j < have && keep; j++) {
-        if (dec_hash[dbase + j] == h && dec_len[dbase + j] == L) {
-          bool eq = true;
-          for (uint32_t i = 0; i < L; i++) if (dec_rows[md_dec_byte(n_slots, dbase + j, i)] != mine[i]) { eq = false; break; }
-          if (eq) keep = false;
-        }
-      }
-      for (uint32_t j = 0; j < a && keep; j++) {
-        if (s_hash[j] == h && A.len[a0 + j] == L) {
-          const uint8_t* o = A.rows + (uint64_t)(a0 + j) * MD_DECOY_ROW; bool eq = true;
-          for (uint32_t i = 0; i < L; i++) if (o[i] != mine[i]) { eq = false; break; }
-          if (eq) keep = false;
-        }
-      }
-    }
-    s_keep[a] = keep ? 1 : 0;
-  }
-  __syncthreads();
-  // ordered compaction: thread t owns the contiguous chunk [t*per, (t+1)*per)
-  const uint32_t per = (na + blockDim.x - 1) / blockDim.x;
-  const uint32_t b = threadIdx.x * per, e = min(b + per, na);
-  uint32_t c = 0;
-  for (uint32_t a = b; a < e; a++) c += s_keep[a];
-  s_scan[threadIdx.x] = c;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    uint32_t run = 0;
-    for (uint32_t t = 0; t < blockDim.x; t++) { uint32_t v = s_scan[t]; s_scan[t] = run; run += v; }
-    s_base = run;
-  }
-  __syncthreads();
-  uint32_t o = have + s_scan[threadIdx.x];
-  for (uint32_t a = b; a < e; a++) {
-    if (!s_keep[a]) continue;
-    if (o < n_per) {
-      const uint64_t src = a0 + a, dst = dbase + o;
-      const uint4* sr = reinterpret_cast<const uint4*>(A.rows + src * MD_DECOY_ROW);
-      for (uint32_t q = 0; q < 4; q++) *reinterpret_cast<uint4*>(dec_rows + md_dec_byte(n_slots, dst, q * 16u)) = sr[q];
-      dec_len[dst] = A.len[src]; dec_mask[dst] = A.mask[src]; dec_w[dst] = A.w[src]; dec_hash[dst] = s_hash[a];
-      dec_attempt[dst] = att_base[li] + a;
-    }
-    o++;
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) dec_count[s] = min(n_per, have + s_base);
-}
-
+// the repair kernel of a vmode (see k_decoy_random)
 template <class MaskT>
-void launch_random(md_ctx* ctx, int vmode, uint32_t grid, const RepairArgs& RA, const DecoyTables& T, const AttemptOut& O) {
-  if (vmode == 0) MD_LAUNCH(ctx, (k_decoy_random<0, MaskT>), grid, kThreads, 0, RA, ctx->mods, T, O);
-  else if (vmode == 1) MD_LAUNCH(ctx, (k_decoy_random<1, MaskT>), grid, kThreads, 0, RA, ctx->mods, T, O);
-  else MD_LAUNCH(ctx, (k_decoy_random<2, MaskT>), grid, kThreads, 0, RA, ctx->mods, T, O);
-}
+auto random_kernel(int vmode) { return vmode == 0 ? k_decoy_random<0, MaskT> : vmode == 1 ? k_decoy_random<1, MaskT> : k_decoy_random<2, MaskT>; }
 template <class MaskT>
 int random_occupancy(int vmode) {
   static int cached[3] = {0, 0, 0};     // (a property of the kernel image: queried once per process)
-  if (cached[vmode]) return cached[vmode];
-  int occ = 0;
-  if (vmode == 0) MD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_decoy_random<0, MaskT>, kThreads, 0));
-  else if (vmode == 1) MD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_decoy_random<1, MaskT>, kThreads, 0));
-  else MD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_decoy_random<2, MaskT>, kThreads, 0));
-  cached[vmode] = occ > 0 ? occ : 1;
+  if (!cached[vmode]) {
+    int occ = 0;
+    MD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, random_kernel<MaskT>(vmode), kThreads, 0));
+    cached[vmode] = occ > 0 ? occ : 1;
+  }
   return cached[vmode];
 }
 
@@ -978,20 +902,19 @@ DecoyTables make_tables(const ModTables& M) {
   memset(&T, 0, sizeof(T));
   const char* alpha = MD_ALPHABET;
   struct E { int64_t m; int a; };
-  std::vector<E> v;
+  std::vector<E> v;   // the letters by mprime ascending, ties by alphabet index
   for (int a = 0; a < MD_ALPHABET_SIZE; a++) {
     uint32_t code = md_code_of((uint8_t)alpha[a]);
     T.code_of_a[a] = (uint8_t)code;
-    T.has_fix_a[a] = M.has_fix[code]; T.has_var_a[a] = M.has_var[code]; T.var_a[a] = M.var[code];
+    T.var_a[a] = M.var[code];
     T.mprime[a] = M.mass[code] + (M.has_fix[code] ? M.fix[code] : 0);
     v.push_back({T.mprime[a], a});
   }
   std::sort(v.begin(), v.end(), [](const E& x, const E& y) { return x.m != y.m ? x.m < y.m : x.a < y.a; });
-  for (int k = 0; k < 32; k++) { T.sorted_m[k] = INT64_MAX; T.sorted_a[k] = 255; T.run_min_a[k] = 255; }
-  for (int k = 0; k < MD_ALPHABET_SIZE; k++) { T.sorted_m[k] = v[k].m; T.sorted_a[k] = (uint8_t)v[k].a; }
+  uint8_t run_min[MD_ALPHABET_SIZE];   // lowest alphabet index among the letters of equal mass, at each sorted position
   for (int k = 0; k < MD_ALPHABET_SIZE; k++) {
     int j = k; while (j > 0 && v[j - 1].m == v[k].m) j--;  // first of the equal-mass run has the lowest alphabet index
-    T.run_min_a[k] = (uint8_t)v[j].a;
+    run_min[k] = (uint8_t)v[j].a;
   }
   // gap tables
   {
@@ -1034,7 +957,7 @@ DecoyTables make_tables(const ModTables& M) {
   {
     int n = 0; int64_t u[32]; uint8_t rep[32];
     for (int k = 0; k < MD_ALPHABET_SIZE; k++)
-      if (n == 0 || v[k].m != u[n - 1]) { u[n] = v[k].m; rep[n] = T.run_min_a[k]; n++; }
+      if (n == 0 || v[k].m != u[n - 1]) { u[n] = v[k].m; rep[n] = run_min[k]; n++; }
     for (int j = 0; j < 32; j++) { T.nn_thr2[j] = INT32_MAX; T.nn_letter[j] = j < n ? rep[j] : rep[n - 1]; }
     for (int j = 0; j + 1 < n; j++) T.nn_thr2[j] = (int32_t)(u[j] + u[j + 1] - (rep[j] < rep[j + 1] ? 0 : 1));
     T.nn_lo = (int32_t)(u[0] - 1); T.nn_hi = (int32_t)(u[n - 1] + 1);
@@ -1048,6 +971,160 @@ DecoyTables make_tables(const ModTables& M) {
     }
   }
   return T;
+}
+
+// Spectra in (roughly) ascending precursor mass: neighbouring attempts grow sequences of similar length (lockstep passes).
+// (The order only steers which attempts run side by side, not the results: a counting sort into 4096 mass buckets is
+// as good as an exact sort and costs microseconds instead of half a millisecond of host time per call.)
+std::vector<uint32_t> mass_order(const std::vector<md_precursor>& prec) {
+  const uint32_t n = (uint32_t)prec.size();
+  int64_t mlo = INT64_MAX, mhi = INT64_MIN;
+  for (uint32_t s = 0; s < n; s++) { mlo = std::min(mlo, prec[s].mass); mhi = std::max(mhi, prec[s].mass); }
+  constexpr uint32_t kBuckets = 4096;
+  const double scale = mhi > mlo ? (double)(kBuckets - 1) / (double)(mhi - mlo) : 0.0;
+  std::vector<uint32_t> head(kBuckets + 1, 0), bucket(n), order(n);
+  for (uint32_t s = 0; s < n; s++) { bucket[s] = (uint32_t)((double)(prec[s].mass - mlo) * scale); head[bucket[s] + 1]++; }
+  for (uint32_t b = 0; b < kBuckets; b++) head[b + 1] += head[b];
+  for (uint32_t s = 0; s < n; s++) order[head[bucket[s]]++] = s;
+  return order;
+}
+
+// The work items of one round: list entries of (spectrum, consecutive attempt ordinals), level by level.
+struct RoundPlan {
+  std::vector<uint32_t> list, off, base;   // per entry: spectrum, prefix of attempt counts (one more), first attempt ordinal
+  std::vector<uint32_t> blk;               // coarse index into off (find_entry_coarse)
+  uint32_t level_begin[kRoundLevels + 1] = {};
+};
+
+// How many attempts each unfinished spectrum gets in this round (count: its decoys so far; used: its attempts so far, of at
+// most cap; visited in `order`).  A spectrum's decoys are its first n distinct successes in attempt order, so asking for too
+// many only wastes work; asking for too few costs another round, and a round never takes less than one 100-try attempt
+// (~0.3 ms) however small it is.  Round 0 asks for want0_pct % of the n still missing + 32; later rounds use the spectrum's
+// own yield with later_factor head room (their attempts are the expensive ones: hard spectra), and rounds too small to fill
+// the GPU ask for up to 4x that.  No entries: every spectrum has its decoys or has used up its attempts.
+RoundPlan plan_round(const std::vector<uint32_t>& count, const std::vector<uint32_t>& used, const std::vector<uint32_t>& cap,
+                     const std::vector<uint32_t>& order, uint32_t n_per, int round, uint32_t want0_pct, double later_factor) {
+  std::vector<uint32_t> wants, todo;
+  uint64_t sum = 0;
+  for (const uint32_t s : order) {
+    if (count[s] >= n_per || used[s] >= cap[s]) continue;
+    uint32_t want;
+    if (used[s] == 0) { const uint32_t rem = n_per - count[s]; want = (uint32_t)((uint64_t)rem * want0_pct / 100u) + 32; }
+    else {
+      double yield = std::max(0.02, (double)count[s] / (double)used[s]);
+      want = (uint32_t)((double)(n_per - count[s]) / yield * later_factor) + 48;
+    }
+    want = std::min<uint32_t>({want, (uint32_t)(kMaxRoundAttempts * kRoundLevels), cap[s] - used[s]});
+    todo.push_back(s); wants.push_back(want); sum += want;
+  }
+  const double boost = round == 0 || sum == 0 ? 1.0 : std::min(4.0, std::max(1.0, 300000.0 / (double)sum));
+  // A list entry is at most kMaxRoundAttempts attempts of one spectrum (the selection kernel's table); a spectrum that gets
+  // more this round -- the hard ones, which would otherwise need a round per 4096 attempts, each round as long as its slowest
+  // attempt however few attempts it has -- has several entries with consecutive attempt ordinals.  The list holds every
+  // spectrum's first entry, then the second entries, ...: k_decoy_select runs once per level, in that order.
+  struct Entry { uint32_t s, n, base; };
+  std::vector<Entry> level[kRoundLevels];
+  uint64_t planned = 0;
+  for (size_t i = 0; i < todo.size(); i++) {
+    const uint32_t s = todo[i];
+    const uint32_t want = std::min<uint32_t>({(uint32_t)((double)wants[i] * boost), (uint32_t)(kMaxRoundAttempts * kRoundLevels), cap[s] - used[s]});
+    if (planned + want > 0x7FFFFFFFull) break;  // the rest waits for the next round
+    planned += want;
+    for (uint32_t c = 0, done = 0; done < want; c++) {
+      const uint32_t chunk = std::min<uint32_t>(want - done, (uint32_t)kMaxRoundAttempts);
+      level[c].push_back(Entry{s, chunk, used[s] + done});
+      done += chunk;
+    }
+  }
+  RoundPlan R;
+  R.off.assign(1, 0);
+  for (int c = 0; c < kRoundLevels; c++) {
+    R.level_begin[c] = (uint32_t)R.list.size();
+    for (const Entry& e : level[c]) { R.list.push_back(e.s); R.base.push_back(e.base); R.off.push_back(R.off.back() + e.n); }
+  }
+  R.level_begin[kRoundLevels] = (uint32_t)R.list.size();
+  if (R.list.empty()) return R;
+  // coarse index: entry of every 1024th work item (+ one past the end)
+  const uint32_t n_list = (uint32_t)R.list.size(), total = R.off.back(), nb = (total >> kBlkLog) + 2;
+  R.blk.resize(nb);
+  for (uint32_t b = 0, e = 0; b < nb; b++) {
+    const uint64_t w0 = std::min<uint64_t>((uint64_t)b << kBlkLog, total - 1);
+    while (e + 1 < n_list && R.off[e + 1] <= w0) e++;
+    R.blk[b] = e;
+  }
+  return R;
+}
+
+// The attempt kernels of one round: every work item of RA becomes one row of O (len 0: no decoy).  Returns whether
+// ctx->ev_trace holds the round's per-kernel times.
+bool launch_attempts(md_ctx* ctx, int mode, int vmode, bool wide_only, const RandomArgs& RA, const DecoyTables& T, const AttemptOut& O,
+                     const PeptideView& PV) {
+  IdentifyWorkspace& W = ctx->ws;
+  const uint32_t total = RA.total;
+  if (mode == MD_DECOY_PERMUTE_TARGET) {
+    MD_LAUNCH(ctx, k_decoy_permute, blocks(total, kThreads), kThreads, 0, RA, T, W.cand_off.p, W.cand_desc.p, W.cand_mask.p, W.cand_w.p, ctx->index.rows.p,
+              O, PV, ctx->mods);
+    return false;
+  }
+  if (ctx->mods.has_terminal) {
+    MD_LAUNCH(ctx, k_decoy_random_terminal, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * 8u), kThreads, 0, RA, ctx->mods, T, O, PV);
+    return false;
+  }
+  // grow every attempt; repair those up to 32 residues with 32-bit position masks, then the longer ones with 64-bit
+  // masks; finish the hits.  The two lists keep the work-item order (spectra by mass: neighbouring lanes repair
+  // sequences of similar length).
+  const size_t tpad = ((size_t)total + 15) & ~(size_t)15;
+  W.t_grown.need(2 * (size_t)total + 2); W.t_start.need(4 * (size_t)total + 4); W.t_route.need(2 * tpad); W.t_narrow.need((size_t)total + 1);
+  W.t_wide.need((size_t)total + 1);
+  GrownAttempt* grown = reinterpret_cast<GrownAttempt*>(W.t_grown.p);
+  StartState* start = reinterpret_cast<StartState*>(W.t_start.p);
+  uint8_t* to_narrow = W.t_route.p; uint8_t* to_wide = W.t_route.p + tpad;
+  uint32_t* queue = W.t_queue.p;
+  // (MD_TRACE: an event behind each step, printed with the round's line)
+  auto trace_ev = [&](int i) { if (ctx->trace) MD_CUDA(cudaEventRecord(ctx->ev_trace[i], ctx->stream)); };
+  MD_CUDA(cudaMemsetAsync(queue, 0, 4 * sizeof(uint32_t), ctx->stream));
+  trace_ev(0);
+  MD_LAUNCH(ctx, k_decoy_grow, blocks(total, kGrowThreads), kGrowThreads, 0, RA, T, O, grown, start, to_narrow, to_wide, wide_only ? 0u : 32u);
+  trace_ev(1);
+  cubx_select_flagged_index(ctx, to_narrow, W.t_narrow.p, queue + 1, total);
+  cubx_select_flagged_index(ctx, to_wide, W.t_wide.p, queue + 3, total);
+  trace_ev(2);
+  const auto narrow = random_kernel<uint32_t>(vmode), wide = random_kernel<uint64_t>(vmode);
+  const uint32_t grid = (total + kThreads - 1) / kThreads;
+  if (!wide_only)
+    MD_LAUNCH(ctx, narrow, std::min<uint32_t>(grid, (uint32_t)ctx->n_sm * (uint32_t)random_occupancy<uint32_t>(vmode)), kThreads, 0,
+              (RepairArgs{W.t_narrow.p, queue + 1, queue, grown, start, RA.seed, RA.overflow}), ctx->mods, T, O);
+  trace_ev(3);
+  MD_LAUNCH(ctx, wide, std::min<uint32_t>(grid, (uint32_t)ctx->n_sm * (uint32_t)random_occupancy<uint64_t>(vmode)), kThreads, 0,
+            (RepairArgs{W.t_wide.p, queue + 3, queue + 2, grown, start, RA.seed, RA.overflow}), ctx->mods, T, O);
+  trace_ev(4);
+  MD_LAUNCH(ctx, k_decoy_finish, blocks(total, 256), 256, 0, total, T, O, grown, PV);
+  trace_ev(5);
+  return ctx->trace;
+}
+
+// k_decoy_select once per level of the round, in level order (a spectrum's later entries see what its earlier ones kept),
+// through the hash set when it fits shared memory, else the exact scan.
+void launch_selects(md_ctx* ctx, const RoundPlan& R, const std::vector<uint32_t>& count, int round, uint32_t n, uint32_t n_per, const AttemptOut& O) {
+  IdentifyWorkspace& W = ctx->ws;
+  const DecoyOut D{W.dec_rows.p, W.dec_len.p, W.dec_mask.p, W.dec_w.p, W.dec_hash.p, W.dec_attempt.p, W.dec_count.p, (uint64_t)n * n_per};
+  for (int c = 0; c < kRoundLevels; c++) {
+    const uint32_t lb = R.level_begin[c], le = R.level_begin[c + 1];
+    if (lb == le) continue;
+    uint32_t need = 1, max_na = 1;                        // most (accepted + attempted) / attempted of one entry of this level
+    for (uint32_t i = lb; i < le; i++) {
+      const uint32_t na = R.off[i + 1] - R.off[i];
+      need = std::max(need, std::min(n_per, count[R.list[i]] + c * (uint32_t)kMaxRoundAttempts) + na); max_na = std::max(max_na, na);
+    }
+    uint32_t slots = 1024; while ((uint64_t)slots * 3 < (uint64_t)need * 4) slots <<= 1;   // load factor <= 0.75 even if every attempt succeeded
+    max_na = (max_na + 7u) & ~7u;
+    const bool hashed = (size_t)slots * 12 + (size_t)max_na * 10 <= (size_t)(MD_SELECT_SMEM_MAX);
+    if (!hashed) slots = 0;                                // the exact scan: hashes and kept list only
+    const size_t smem = (size_t)slots * 12 + (size_t)max_na * 10;
+    if (ctx->trace) fprintf(stderr, "[md_trace]   decoy select round %d level %d: entries=%u kernel=%s\n", round, c, le - lb, hashed ? "hash" : "n2");
+    MD_CUDA(cudaFuncSetAttribute(k_decoy_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    MD_LAUNCH(ctx, k_decoy_select, le - lb, 256, smem, W.t_list.p + lb, W.t_off.p + lb, W.t_base.p + lb, n_per, slots, max_na, O, D);
+  }
 }
 
 }  // namespace
@@ -1073,198 +1150,64 @@ void decoys_generate_dev(md_ctx* ctx, uint32_t n, uint32_t n_per, int mode, uint
       MD_REQUIRE(T.mprime[a] > 0 && T.mprime[a] < (1 << 29) && T.var_a[a] > -(1 << 29) && T.var_a[a] < (1 << 29), MD_ERR_UNSUPPORTED,
                  "decoy generation works in 32-bit residuals: residue and modification masses must stay below 536 Da");
   PeptideView PV{(const unsigned long long*)P.ht_key.p, P.ht_val.p, P.ht_mask, P.seq.p, P.seq_off.p, P.len.p};
-  std::vector<uint64_t> h_cand_off;
-  if (mode == MD_DECOY_PERMUTE_TARGET) {
-    h_cand_off.resize(n + 1);
-    MD_CUDA(cudaMemcpyAsync(h_cand_off.data(), W.cand_off.p, (n + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    MD_CUDA(cudaStreamSynchronize(ctx->stream));
-  }
-  // per spectrum bookkeeping on the host
-  std::vector<uint32_t> used(n, 0), count(n, 0), cap(n);
   // stored decoys come first (tasks/identification.rs:259-283); only the remainder is generated
-  if (mode == MD_DECOY_REFERENCE_RANDOM && ctx->dindex.ready && ctx->dindex.n > 0) {
-    decoys_reuse_dev(ctx, n, n_per);
-    MD_CUDA(cudaMemcpyAsync(count.data(), W.dec_count.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    MD_CUDA(cudaStreamSynchronize(ctx->stream));
-  }
-  // spectra in (roughly) ascending precursor mass: neighbouring attempts grow sequences of similar length (lockstep passes)
-  std::vector<uint32_t> by_mass(n);
-  {
-    std::vector<md_precursor> hp(n);
-    MD_CUDA(cudaMemcpyAsync(hp.data(), W.prec.p, n * sizeof(md_precursor), cudaMemcpyDeviceToHost, ctx->stream));
-    MD_CUDA(cudaStreamSynchronize(ctx->stream));
-    // (the order only steers which attempts run side by side, not the results: a counting sort into 4096 mass buckets is
-    // as good as an exact sort and costs microseconds instead of half a millisecond of host time per call)
-    int64_t mlo = INT64_MAX, mhi = INT64_MIN;
-    for (uint32_t s = 0; s < n; s++) { mlo = std::min(mlo, hp[s].mass); mhi = std::max(mhi, hp[s].mass); }
-    constexpr uint32_t kBuckets = 4096;
-    const double scale = mhi > mlo ? (double)(kBuckets - 1) / (double)(mhi - mlo) : 0.0;
-    std::vector<uint32_t> head(kBuckets + 1, 0), bucket(n);
-    for (uint32_t s = 0; s < n; s++) { bucket[s] = (uint32_t)((double)(hp[s].mass - mlo) * scale); head[bucket[s] + 1]++; }
-    for (uint32_t b = 0; b < kBuckets; b++) head[b + 1] += head[b];
-    for (uint32_t s = 0; s < n; s++) by_mass[head[bucket[s]]++] = s;
-  }
+  const bool stored = mode == MD_DECOY_REFERENCE_RANDOM && ctx->dindex.ready && ctx->dindex.n > 0;
+  if (stored) decoys_reuse_dev(ctx, n, n_per);
+  // per spectrum bookkeeping on the host: decoys so far, attempts used, attempt cap
+  std::vector<uint32_t> count(n, 0), used(n, 0), cap(n);
+  std::vector<md_precursor> hp(n);
+  std::vector<uint64_t> h_cand_off(mode == MD_DECOY_PERMUTE_TARGET ? n + 1 : 0);
+  MD_CUDA(cudaMemcpyAsync(hp.data(), W.prec.p, n * sizeof(md_precursor), cudaMemcpyDeviceToHost, ctx->stream));
+  if (stored) MD_CUDA(cudaMemcpyAsync(count.data(), W.dec_count.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (!h_cand_off.empty()) MD_CUDA(cudaMemcpyAsync(h_cand_off.data(), W.cand_off.p, (n + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+  MD_CUDA(cudaStreamSynchronize(ctx->stream));
+  const std::vector<uint32_t> by_mass = mass_order(hp);
   for (uint32_t s = 0; s < n; s++) {
     uint64_t c = md_attempt_cap(n_per);
     if (mode == MD_DECOY_PERMUTE_TARGET) c = std::min<uint64_t>(c, (h_cand_off[s + 1] - h_cand_off[s]) * 1000ull);
     cap[s] = (uint32_t)c;
   }
   // how try_variable_modifications runs inside the repair loop (see k_decoy_random)
-  int vmode = 0, occ_narrow = 1, occ_wide = 1;
+  int vmode = 0;
+  bool any_var_letter = false;
+  for (int a = 0; a < MD_ALPHABET_SIZE; a++) any_var_letter |= ctx->mods.has_var[T.code_of_a[a]] != 0;
+  if (ctx->mods.nvar > 0 && any_var_letter)
+    vmode = (ctx->mods.var_simple_code >= 0 && md_alpha_of_code((uint32_t)ctx->mods.var_simple_code) >= 0) ? 1 : 2;
   const bool wide_only = getenv("MD_DECOY_WIDE_ONLY") != nullptr;   // debugging: skip the 32-bit pass
-  if (mode == MD_DECOY_REFERENCE_RANDOM) {
-    bool any_var_letter = false;
-    for (int a = 0; a < MD_ALPHABET_SIZE; a++) any_var_letter |= T.has_var_a[a] != 0;
-    if (ctx->mods.nvar > 0 && any_var_letter)
-      vmode = (ctx->mods.var_simple_code >= 0 && md_alpha_of_code((uint32_t)ctx->mods.var_simple_code) >= 0) ? 1 : 2;
-    occ_narrow = random_occupancy<uint32_t>(vmode); occ_wide = random_occupancy<uint64_t>(vmode);
-  }
-  DevBuf<uint32_t>& d_list = W.t_list; DevBuf<uint32_t>& d_off = W.t_off; DevBuf<uint32_t>& d_base = W.t_base; DevBuf<uint32_t>& d_queue = W.t_queue;
-  DevBuf<int>& d_ovf = W.t_ovf;
-  d_list.need((size_t)n * kRoundLevels + 1); d_off.need((size_t)n * kRoundLevels + 2); d_base.need((size_t)n * kRoundLevels + 1); d_queue.need(4); d_ovf.need(1);
-  MD_CUDA(cudaMemsetAsync(d_ovf.p, 0, sizeof(int), ctx->stream));
-  std::vector<uint32_t> list, off, base, blk;
   const double later_factor = getenv("MD_DECOY_LATER_PCT") ? std::max(100, atoi(getenv("MD_DECOY_LATER_PCT"))) / 100.0 : 1.05;   // head room of the later rounds (swept on C2: 100..180 %)
   const uint32_t want0_pct = getenv("MD_DECOY_WANT0_PCT") ? (uint32_t)std::max(100, atoi(getenv("MD_DECOY_WANT0_PCT"))) : 110u;   // round 0 asks for n * 1.10 + 32 attempts (swept on C2: 100..160 %)
+  W.t_list.need((size_t)n * kRoundLevels + 1); W.t_off.need((size_t)n * kRoundLevels + 2); W.t_base.need((size_t)n * kRoundLevels + 1); W.t_queue.need(4); W.t_ovf.need(1);
+  MD_CUDA(cudaMemsetAsync(W.t_ovf.p, 0, sizeof(int), ctx->stream));
   for (int round = 0;; round++) {   // until every spectrum has its decoys or has used up its attempts (every round makes progress)
-    list.clear(); off.assign(1, 0); base.clear();
-    // How many attempts each unfinished spectrum gets this round.  A spectrum's decoys are its first n distinct successes
-    // in attempt order, so asking for too many only wastes work; asking for too few costs another round, and a round
-    // never takes less than one 100-try attempt (~0.3 ms) however small it is.  Round 0 asks for 1.1 n + 32; later rounds use
-    // the spectrum's own yield with 5 % head room (their attempts are the expensive ones: hard spectra), and rounds too small to fill the GPU ask for up to 4x that.
-    std::vector<uint32_t> wants, todo;
-    uint64_t sum = 0;
-    for (uint32_t si = 0; si < n; si++) {
-      const uint32_t s = by_mass[si];
-      if (count[s] >= n_per || used[s] >= cap[s]) continue;
-      uint32_t want;
-      if (used[s] == 0) { const uint32_t rem = n_per - count[s]; want = (uint32_t)((uint64_t)rem * want0_pct / 100u) + 32; }
-      else {
-        double yield = std::max(0.02, (double)count[s] / (double)used[s]);
-        want = (uint32_t)((double)(n_per - count[s]) / yield * later_factor) + 48;
-      }
-      want = std::min<uint32_t>({want, (uint32_t)(kMaxRoundAttempts * kRoundLevels), cap[s] - used[s]});
-      todo.push_back(s); wants.push_back(want); sum += want;
-    }
-    const double boost = round == 0 || sum == 0 ? 1.0 : std::min(4.0, std::max(1.0, 300000.0 / (double)sum));
-    // A list entry is at most kMaxRoundAttempts attempts of one spectrum (the selection kernel's table); a spectrum that gets
-    // more this round -- the hard ones, which would otherwise need a round per 4096 attempts, each round as long as its slowest
-    // attempt however few attempts it has -- has several entries with consecutive attempt ordinals.  The list holds every
-    // spectrum's first entry, then the second entries, ...: k_decoy_select runs once per level, in that order.
-    struct Entry { uint32_t s, n, base; };
-    std::vector<Entry> level[kRoundLevels];
-    uint64_t planned = 0;
-    for (size_t i = 0; i < todo.size(); i++) {
-      const uint32_t s = todo[i];
-      const uint32_t want = std::min<uint32_t>({(uint32_t)((double)wants[i] * boost), (uint32_t)(kMaxRoundAttempts * kRoundLevels), cap[s] - used[s]});
-      if (planned + want > 0x7FFFFFFFull) break;  // the rest waits for the next round
-      planned += want;
-      for (uint32_t c = 0, done = 0; done < want; c++) {
-        const uint32_t chunk = std::min<uint32_t>(want - done, (uint32_t)kMaxRoundAttempts);
-        level[c].push_back(Entry{s, chunk, used[s] + done});
-        done += chunk;
-      }
-    }
-    uint32_t level_begin[kRoundLevels + 1];
-    for (int c = 0; c < kRoundLevels; c++) {
-      level_begin[c] = (uint32_t)list.size();
-      for (const Entry& e : level[c]) { list.push_back(e.s); base.push_back(e.base); off.push_back(off.back() + e.n); }
-    }
-    level_begin[kRoundLevels] = (uint32_t)list.size();
-    if (list.empty()) break;
-    const uint32_t n_list = (uint32_t)list.size(), total = off.back();
-    bool split = false;    // ev_trace holds this round's per-kernel times
+    const RoundPlan R = plan_round(count, used, cap, by_mass, n_per, round, want0_pct, later_factor);
+    if (R.list.empty()) break;
+    const uint32_t n_list = (uint32_t)R.list.size(), total = R.off.back(), nb = (uint32_t)R.blk.size();
     W.att_rows.need((size_t)total * MD_DECOY_ROW + 64); W.att_len.need(total + 1); W.att_mask.need(total + 1); W.att_w.need(total + 1); W.att_hash.need(total + 1);
-    AttemptOut O{W.att_rows.p, W.att_len.p, W.att_mask.p, W.att_w.p, W.att_hash.p};
-    MD_CUDA(cudaMemcpyAsync(d_list.p, list.data(), n_list * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-    MD_CUDA(cudaMemcpyAsync(d_off.p, off.data(), (n_list + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-    MD_CUDA(cudaMemcpyAsync(d_base.p, base.data(), n_list * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    W.t_blk.need(nb);
+    const AttemptOut O{W.att_rows.p, W.att_len.p, W.att_mask.p, W.att_w.p, W.att_hash.p};
+    MD_CUDA(cudaMemcpyAsync(W.t_list.p, R.list.data(), n_list * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    MD_CUDA(cudaMemcpyAsync(W.t_off.p, R.off.data(), (n_list + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    MD_CUDA(cudaMemcpyAsync(W.t_base.p, R.base.data(), n_list * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    MD_CUDA(cudaMemcpyAsync(W.t_blk.p, R.blk.data(), nb * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
     MD_CUDA(cudaEventRecord(ctx->ev[4], ctx->stream));
-    if (mode == MD_DECOY_REFERENCE_RANDOM) {
-      RandomArgs RA;
-      {   // coarse index: entry of every 1024th work item (+ one past the end)
-        const uint32_t nb = (total >> kBlkLog) + 2;
-        blk.resize(nb);
-        uint32_t e = 0;
-        for (uint32_t b = 0; b < nb; b++) {
-          const uint64_t w0 = std::min<uint64_t>((uint64_t)b << kBlkLog, total - 1);
-          while (e + 1 < n_list && off[e + 1] <= w0) e++;
-          blk[b] = e;
-        }
-        W.t_blk.need(nb);
-        MD_CUDA(cudaMemcpyAsync(W.t_blk.p, blk.data(), nb * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-      }
-      RA.prec = W.prec.p; RA.list = d_list.p; RA.att_off = d_off.p; RA.att_base = d_base.p; RA.n_list = n_list; RA.total = total; RA.att_blk = W.t_blk.p;
-      RA.seed = seed; RA.overflow = d_ovf.p;
-      if (ctx->mods.has_terminal) {
-        MD_LAUNCH(ctx, k_decoy_random_terminal, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * 8u), kThreads, 0, RA, ctx->mods, T, O, PV);
-      } else {
-        // grow every attempt; repair those up to 32 residues with 32-bit position masks, then the longer ones with 64-bit
-        // masks; finish the hits.  The two lists keep the work-item order (spectra by mass: neighbouring lanes repair
-        // sequences of similar length).
-        const size_t tpad = ((size_t)total + 15) & ~(size_t)15;
-        W.t_grown.need(2 * (size_t)total + 2); W.t_start.need(4 * (size_t)total + 4); W.t_route.need(2 * tpad); W.t_narrow.need((size_t)total + 1);
-        W.t_wide.need((size_t)total + 1);
-        GrownAttempt* grown = reinterpret_cast<GrownAttempt*>(W.t_grown.p);
-        StartState* start = reinterpret_cast<StartState*>(W.t_start.p);
-        uint8_t* to_narrow = W.t_route.p; uint8_t* to_wide = W.t_route.p + tpad;
-        // (MD_TRACE: an event behind each step, printed with the round's line)
-        auto trace_ev = [&](int i) { if (ctx->trace) MD_CUDA(cudaEventRecord(ctx->ev_trace[i], ctx->stream)); };
-        MD_CUDA(cudaMemsetAsync(d_queue.p, 0, 4 * sizeof(uint32_t), ctx->stream));
-        trace_ev(0);
-        MD_LAUNCH(ctx, k_decoy_grow, blocks(total, kGrowThreads), kGrowThreads, 0, RA, T, O, grown, start, to_narrow, to_wide, wide_only ? 0u : 32u);
-        trace_ev(1);
-        cubx_select_flagged_index(ctx, to_narrow, W.t_narrow.p, d_queue.p + 1, total);
-        cubx_select_flagged_index(ctx, to_wide, W.t_wide.p, d_queue.p + 3, total);
-        trace_ev(2);
-        RepairArgs R{W.t_narrow.p, d_queue.p + 1, d_queue.p, grown, start, seed, d_ovf.p};
-        if (!wide_only) launch_random<uint32_t>(ctx, vmode, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * (uint32_t)occ_narrow), R, T, O);
-        trace_ev(3);
-        R = RepairArgs{W.t_wide.p, d_queue.p + 3, d_queue.p + 2, grown, start, seed, d_ovf.p};
-        launch_random<uint64_t>(ctx, vmode, std::min<uint32_t>((total + kThreads - 1) / kThreads, (uint32_t)ctx->n_sm * (uint32_t)occ_wide), R, T, O);
-        trace_ev(4);
-        MD_LAUNCH(ctx, k_decoy_finish, blocks(total, 256), 256, 0, total, T, O, grown, PV);
-        trace_ev(5);
-        split = ctx->trace;
-      }
-    } else {
-      MD_LAUNCH(ctx, k_decoy_permute, blocks(total, kThreads), kThreads, 0, W.prec.p, d_list.p, d_off.p, d_base.p, n_list, total, seed, T, W.cand_off.p,
-                W.cand_desc.p, W.cand_mask.p, W.cand_w.p, ctx->index.rows.p, O, PV, ctx->mods);
-    }
+    const RandomArgs RA{W.prec.p, W.t_list.p, W.t_off.p, W.t_base.p, W.t_blk.p, total, seed, W.t_ovf.p};
+    const bool split = launch_attempts(ctx, mode, vmode, wide_only, RA, T, O, PV);
     MD_CUDA(cudaEventRecord(ctx->ev[5], ctx->stream));
     ctx->mark("  attempts");
-    for (int c = 0; c < kRoundLevels; c++) {
-      const uint32_t lb = level_begin[c], le = level_begin[c + 1];
-      if (lb == le) continue;
-      uint32_t need = 1, max_na = 1;                        // most (accepted + attempted) / attempted of one entry of this level
-      for (uint32_t i = lb; i < le; i++) { need = std::max(need, std::min(n_per, count[list[i]] + c * (uint32_t)kMaxRoundAttempts) + (off[i + 1] - off[i])); max_na = std::max(max_na, off[i + 1] - off[i]); }
-      uint32_t slots = 1024; while ((uint64_t)slots * 3 < (uint64_t)need * 4) slots <<= 1;   // load factor <= 0.75 even if every attempt succeeded
-      max_na = (max_na + 7u) & ~7u;
-      const size_t smem = (size_t)slots * 12 + (size_t)max_na * 10;
-      const bool hashed = smem <= (size_t)(MD_SELECT_SMEM_MAX);
-      if (ctx->trace) fprintf(stderr, "[md_trace]   decoy select round %d level %d: entries=%u kernel=%s\n", round, c, le - lb, hashed ? "hash" : "n2");
-      if (hashed) {
-        MD_CUDA(cudaFuncSetAttribute(k_decoy_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        MD_LAUNCH(ctx, k_decoy_select, le - lb, 256, smem, d_list.p + lb, d_off.p + lb, d_base.p + lb, n_per, slots, max_na, O, (uint64_t)n * n_per, W.dec_rows.p, W.dec_len.p, W.dec_mask.p,
-                  W.dec_w.p, W.dec_hash.p, W.dec_attempt.p, W.dec_count.p);
-      } else {
-        MD_LAUNCH(ctx, k_decoy_select_n2, le - lb, 256, 0, d_list.p + lb, d_off.p + lb, d_base.p + lb, n_per, O, (uint64_t)n * n_per, W.dec_rows.p, W.dec_len.p, W.dec_mask.p, W.dec_w.p,
-                  W.dec_hash.p, W.dec_attempt.p, W.dec_count.p);
-      }
-    }
+    launch_selects(ctx, R, count, round, n, n_per, O);
     MD_CUDA(cudaMemcpyAsync(count.data(), W.dec_count.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
     MD_CUDA(cudaStreamSynchronize(ctx->stream));
     ctx->mark("  select");
-    for (uint32_t i = 0; i < n_list; i++) used[list[i]] += off[i + 1] - off[i];
-    { float ms = 0; cudaEventElapsedTime(&ms, ctx->ev[4], ctx->ev[5]); ctx->acc_ms_kdecoy += ms; ctx->acc_attempts += total;
-      if (ctx->trace) fprintf(stderr, "[md_trace]   decoy round %d: spectra=%u attempts=%u kernel=%.3f ms\n", round, n_list, total, ms);
-      if (split) {
-        float t[5];
-        for (int i = 0; i < 5; i++) MD_CUDA(cudaEventElapsedTime(&t[i], ctx->ev_trace[i], ctx->ev_trace[i + 1]));
-        fprintf(stderr, "[md_trace]   decoy round %d kernels: grow=%.3f lists=%.3f narrow=%.3f wide=%.3f finish=%.3f ms\n", round, t[0], t[1], t[2], t[3], t[4]);
-      } }
+    for (uint32_t i = 0; i < n_list; i++) used[R.list[i]] += R.off[i + 1] - R.off[i];
+    float ms = 0; cudaEventElapsedTime(&ms, ctx->ev[4], ctx->ev[5]); ctx->acc_ms_kdecoy += ms; ctx->acc_attempts += total;
+    if (ctx->trace) fprintf(stderr, "[md_trace]   decoy round %d: spectra=%u attempts=%u kernel=%.3f ms\n", round, n_list, total, ms);
+    if (split) {
+      float t[5];
+      for (int i = 0; i < 5; i++) MD_CUDA(cudaEventElapsedTime(&t[i], ctx->ev_trace[i], ctx->ev_trace[i + 1]));
+      fprintf(stderr, "[md_trace]   decoy round %d kernels: grow=%.3f lists=%.3f narrow=%.3f wide=%.3f finish=%.3f ms\n", round, t[0], t[1], t[2], t[3], t[4]);
+    }
   }
-  const int ovf = d2h_scalar(ctx, d_ovf.p);
+  const int ovf = d2h_scalar(ctx, W.t_ovf.p);
   MD_REQUIRE(ovf != 3, MD_ERR_DEVICE, "decoy generation: internal error (substitution filter disagrees with the mass search)");
   MD_REQUIRE(ovf != 2, MD_ERR_UNSUPPORTED, "decoy generation: |weight - precursor| left the 32-bit range (residue or modification masses above ~1000 Da?)");
   MD_REQUIRE(!ovf, MD_ERR_UNSUPPORTED, "variable-modification placement enumeration exceeds 2^22 subsets for one decoy");

@@ -1,8 +1,14 @@
-// decoyutil.cuh -- device helpers shared by the decoy kernels (decoy.cu, exhaustive.cu).
+// decoyutil.cuh -- device helpers shared by the decoy kernels (decoy.cu, exhaustive.cu, index.cu).
 #pragma once
 #include "common.cuh"
 
 #include <type_traits>
+
+// the accepted decoys of a batch: n_per slots per spectrum, filled from slot 0 up; count = filled slots per spectrum
+struct DecoyOut {
+  uint8_t* rows; uint8_t* len; uint64_t* mask; int64_t* w; uint64_t* hash; uint32_t* attempt; uint32_t* count;
+  uint64_t n_slots;   // decoy slots of the batch (two-plane row layout, md_dec_byte)
+};
 
 struct PeptideView {
   const unsigned long long* ht_key; const uint32_t* ht_val; uint32_t ht_mask;

@@ -21,11 +21,6 @@ struct ExTables {
   uint8_t code_of_a[MD_ALPHABET_SIZE];
 };
 
-struct DecoyOut {
-  uint8_t* rows; uint8_t* len; uint64_t* mask; int64_t* w; uint64_t* hash; uint32_t* attempt; uint32_t* count;
-  uint64_t n_slots;   // decoy slots of the batch (two-plane row layout, md_dec_byte)
-};
-
 __global__ void __launch_bounds__(64) k_decoy_exhaustive(const md_precursor* __restrict__ prec, uint32_t n_spec, uint32_t n_per,
                                                          const __grid_constant__ ExTables T, PeptideView PV, DecoyOut O, int* __restrict__ too_large) {
   const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;

@@ -8,6 +8,7 @@
 // (identification.rs:242-257) then runs on the window's entries, one thread per entry.
 #include "cubx.cuh"
 #include "modpep.cuh"
+#include "decoyutil.cuh"
 
 namespace {
 
@@ -183,9 +184,7 @@ __global__ void k_scatter_candidates(const uint64_t* __restrict__ flat_off, cons
 __global__ void k_scatter_stored_decoys(const uint64_t* __restrict__ flat_off, const uint64_t* __restrict__ rbegin, uint32_t n_spec, uint64_t n_entries,
                                         const uint32_t* __restrict__ flag, const uint32_t* __restrict__ pos, const uint64_t* __restrict__ emask,
                                         const int64_t* __restrict__ ew, const uint32_t* __restrict__ idx_pep, const uint64_t* __restrict__ idx_desc,
-                                        const uint8_t* __restrict__ rows, const uint64_t* __restrict__ store_hash, uint32_t n_per,
-                                        uint64_t n_slots, uint8_t* __restrict__ dec_rows, uint8_t* __restrict__ dec_len, uint64_t* __restrict__ dec_mask,
-                                        int64_t* __restrict__ dec_w, uint64_t* __restrict__ dec_hash, uint32_t* __restrict__ dec_attempt) {
+                                        const uint8_t* __restrict__ rows, const uint64_t* __restrict__ store_hash, uint32_t n_per, DecoyOut D) {
   uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= n_entries || !flag[e]) return;
   uint32_t lo = 0, hi = n_spec;
@@ -198,9 +197,9 @@ __global__ void k_scatter_stored_decoys(const uint64_t* __restrict__ flat_off, c
   const uint8_t* src = rows + (d & 0xFFFFFFFFFFull) * 16;
   const uint32_t L = (uint32_t)(d >> 40) & 0xFF;
   const uint64_t slot = (uint64_t)s * n_per + rank;
-  for (uint32_t k = 0; k < MD_DECOY_ROW; k++) dec_rows[md_dec_byte(n_slots, slot, k)] = k < L ? src[k] : (uint8_t)MD_CODE_OTHER;
-  dec_len[slot] = (uint8_t)L; dec_mask[slot] = emask[e]; dec_w[slot] = ew[e]; dec_hash[slot] = store_hash[idx_pep[i]];
-  dec_attempt[slot] = MD_DECOY_STORED;
+  for (uint32_t k = 0; k < MD_DECOY_ROW; k++) D.rows[md_dec_byte(D.n_slots, slot, k)] = k < L ? src[k] : (uint8_t)MD_CODE_OTHER;
+  D.len[slot] = (uint8_t)L; D.mask[slot] = emask[e]; D.w[slot] = ew[e]; D.hash[slot] = store_hash[idx_pep[i]];
+  D.attempt[slot] = MD_DECOY_STORED;
 }
 
 __global__ void k_stored_counts(const uint64_t* __restrict__ flat_off, const uint32_t* __restrict__ pos, uint32_t n_spec, uint32_t n_per,
@@ -503,8 +502,9 @@ void decoys_reuse_dev(md_ctx* ctx, uint32_t n, uint32_t n_per) {
   uint32_t total = 0;
   const uint64_t E = filter_windows(ctx, X, n, &total);
   if (E) {
+    const DecoyOut D{W.dec_rows.p, W.dec_len.p, W.dec_mask.p, W.dec_w.p, W.dec_hash.p, W.dec_attempt.p, W.dec_count.p, (uint64_t)n * n_per};
     MD_LAUNCH(ctx, k_scatter_stored_decoys, blocks(E), 256, 0, W.flat_off.p, W.rbegin.p, n, E, W.t_flag.p, W.t_pos.p, W.emask.p, W.ew.p, X.pep.p, X.desc.p,
-              X.rows.p, ctx->dstore.hash.p, n_per, (uint64_t)n * n_per, W.dec_rows.p, W.dec_len.p, W.dec_mask.p, W.dec_w.p, W.dec_hash.p, W.dec_attempt.p);
+              X.rows.p, ctx->dstore.hash.p, n_per, D);
   }
   MD_LAUNCH(ctx, k_stored_counts, blocks(n), 256, 0, W.flat_off.p, W.t_pos.p, n, n_per, W.dec_count.p);
   ctx->mark("  reuse");

@@ -2,9 +2,10 @@
 
 The host plans REFERENCE_RANDOM / PERMUTE_TARGET decoys in rounds: every unfinished spectrum gets a budget of attempts,
 split into list entries of at most MD_ROUND_ATTEMPTS (4096) consecutive attempt ordinals, and a select kernel per level
-keeps each spectrum's first distinct successes -- through a shared-memory hash set (k_decoy_select), or, when that set would
-not fit, a quadratic scan (k_decoy_select_n2).  The results must depend on (seed, spectrum_id, attempt) alone: not on the
-entry size, the select kernel, the repair loop's refill constants, the precursor order or the round budgets.
+keeps each spectrum's first distinct successes -- through a shared-memory hash set, or, when that set would not fit, an
+exact quadratic scan (k_decoy_select's two routes, "hash" and "n2" in the trace).  The results must depend on (seed,
+spectrum_id, attempt) alone: not on the entry size, the select route, the repair loop's refill constants, the precursor
+order or the round budgets.
 
 - Test builds of decoy.cu with 64-attempt entries and either 6-bit hashes or the quadratic select (and the repair loop's
   refill threshold, ring size and ring period at their extremes, with the device-side substitution check) run the usual
@@ -37,7 +38,7 @@ VARIANTS = {
     # smallest ring (every lane runs dry) topped up at every step
     "tiny_rounds_hash": ["-DMD_ROUND_ATTEMPTS=64", "-DMD_SELECT_HASH_MASK=0x3Full", "-DMD_REFILL_MIN=1", "-DMD_RNG_RING=4", "-DMD_RNG_PERIOD=1",
                          "-DMD_DECOY_CHECK"],
-    # every level through k_decoy_select_n2; a refill only when the whole warp is free
+    # every level through the exact scan of k_decoy_select; a refill only when the whole warp is free
     "tiny_rounds_n2": ["-DMD_ROUND_ATTEMPTS=64", "-DMD_SELECT_SMEM_MAX=0", "-DMD_REFILL_MIN=32", "-DMD_RNG_RING=16", "-DMD_RNG_PERIOD=5", "-DMD_DECOY_CHECK"],
 }
 VARIANT_KERNEL = {"tiny_rounds_hash": "hash", "tiny_rounds_n2": "n2"}
@@ -205,7 +206,7 @@ def _two_heavy(cpu):
 
 def test_large_counts_take_several_levels_and_quadratic_select(gpu, cpu, capfd):
     """12000 decoys: round 0 asks for 13232 attempts per spectrum, entries of 4096, 4096, 4096 and 944.  Level 0 fits the
-    hash set; levels 1-3 would need more than 220 KB of shared memory and run k_decoy_select_n2.  5000 decoys: two levels,
+    hash set; levels 1-3 would need more than 220 KB of shared memory and run the exact scan.  5000 decoys: two levels,
     both hashed."""
     _setup((gpu, cpu), (synth.CAM,), 0)
     _, pre = _two_heavy(cpu)
